@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's fused sm_100a kernel
     python bench.py --impl reference --gpus N --steps K ...  # the reference's own CPU path, all host cores
+    python bench.py ... --dump-outputs DIR                   # also save what the last timed step computed (sampled envs, .npy)
 
 A "step" = one env.step() of every env of the batch: 30 agents x 65 536 envs per GPU (BASELINE config 3; at N=1
 it is the single-GPU instance of the configuration the metric is quoted on).  Envs are independent, so N GPUs run N
@@ -118,6 +119,25 @@ class ClockSampler(threading.Thread):
                     reasons=sorted(reasons), samples=len(sm))
 
 
+DUMP_BYTES = 60 * 10**6     # all files of one --dump-outputs run, below 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, tag, arrays, budget):
+    """Writes the [E, ...] device arrays of `arrays` as <out_dir>/<tag>_<name>.npy so that two builds can be compared output for
+    output: the same seeded sample of envs for every array (as many as `budget` bytes allow), float64 arrays as float64, all
+    others (integer and bool ones too: their values are exact there) as float32."""
+    import torch
+    arrays = {k: v for k, v in arrays.items() if v is not None}
+    E = next(iter(arrays.values())).shape[0]
+    per_env = sum(t[0].numel() * (8 if t.dtype == torch.float64 else 4) for t in arrays.values())
+    n = max(1, min(E, budget // per_env))
+    pick = np.sort(np.random.RandomState(0).choice(E, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.index_select(0, torch.as_tensor(pick, device=t.device)).cpu().numpy()
+        np.save(os.path.join(out_dir, f"{tag}_{name}.npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
+
+
 def measured_hbm_peak():
     path = os.path.join(REPO, "MEASURED_PEAKS.json")
     if os.path.isfile(path):
@@ -137,25 +157,23 @@ def reference_arm(args, rank, world):
     shapes = load_shapes()
     cores = os.cpu_count() or 1
     procs = max(1, min(cores, args.ref_procs or cores))
+    K = args.steps                          # env.step() calls per env inside the timed region
     if not ref_glue.available():
         # the reference C++ was not compiled here: fall back to the C port of it (never to the product)
         from oracle import oracle as orc
-        t0 = time.perf_counter()
-        res = port_rollouts(orc, shapes, args.n_a, procs, args.ref_envs, args.ref_steps)
-        kind, sample = "port", f"{res['envs']} envs x {args.ref_steps} steps, oracle C port, {procs} OpenMP threads"
-        value, secs = res["value"], time.perf_counter() - t0
+        res = port_rollouts(orc, shapes, args.n_a, procs, args.ref_envs, K)
+        kind, sample = "port", f"{res['envs']} envs x {K} steps, oracle C port, {procs} OpenMP threads"
     else:
-        episodes = min(max(1, (args.steps + 1) // 2), 100)   # a "step" of this arm = 100 env.step() calls per process (bounded sample)
         for _ in range(max(0, min(args.warmup, 1))):
             ref_glue.timed_rollouts(args.n_a, shapes, procs, 1, 20)
-        res = ref_glue.timed_rollouts(args.n_a, shapes, procs, episodes, args.ref_steps)
+        res = ref_glue.timed_rollouts(args.n_a, shapes, procs, 1, K)
         kind = "reference"
-        sample = (f"{procs} processes x {episodes} episodes x {args.ref_steps} steps x {args.n_a} agents, one env each "
+        sample = (f"{procs} processes x {K} steps x {args.n_a} agents, one env each "
                   f"(reference AssemblyEnv.cpp via oracle/_ref + its NumPy glue), env.step() time only")
-        value, secs = res["value"], res["seconds"]
+    value, secs = res["value"], res["seconds"]
     line = {
-        "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
-        "warmup": args.warmup, "ms_per_step": 1e3 * secs / max(1, args.steps), "higher_is_better": True, "scaling": "weak",
+        "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": K,
+        "warmup": args.warmup, "ms_per_step": 1e3 * secs / K, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": {"workload": f"assembly env, {args.n_a} agents, reference CPU path (single env per process; the reference has no vector env)",
                    "n_a": args.n_a, "processes": procs},
@@ -314,6 +332,8 @@ def flocking_line(args, torch, rank, world, local_rank, barrier, max_over_ranks)
     barrier()
     ms = max_over_ranks(ev0.elapsed_time(ev1), device="cuda")
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, "flocking", dict(obs=sim.obs, reward=sim.reward, done=sim.done, p=sim.p, dp=sim.dp), DUMP_BYTES)
     peak, peak_src = measured_hbm_peak()
     b = 8 + 64 + sim.obs_dim * 4 + 4 + 24
     achieved = b * E * n_a / (ms / K * 1e-3) / 1e9
@@ -351,6 +371,9 @@ def predator_prey_line(args, torch, rank, world, local_rank, barrier, max_over_r
     barrier()
     ms = max_over_ranks(ev0.elapsed_time(ev1), device="cuda")
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, "predator_prey", dict(obs=sim.obs, reward=sim.reward, done=sim.done, p=sim.p, dp=sim.dp),
+                     DUMP_BYTES)
     peak, peak_src = measured_hbm_peak()
     b = 8 + 64 + sim.obs_dim * 4 + 4 + 48
     achieved = b * E * n / (ms / K * 1e-3) / 1e9
@@ -387,9 +410,15 @@ def main():
     ap.add_argument("--variant", default="assembly", choices=["assembly", "flocking", "predator_prey"],
                     help="flocking / predator_prey: the variants specified in VARIANTS.md (BASELINE config 5; no reference source, no CPU baseline)")
     ap.add_argument("--ref-procs", type=int, default=0)
-    ap.add_argument("--ref-steps", type=int, default=200)
     ap.add_argument("--ref-envs", type=int, default=256)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of each regime, write what its last step computed (rank 0's envs; a fixed, seeded "
+                         "sample of them) as DIR/<regime or variant>_<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -528,6 +557,11 @@ def main():
             for _ in range(20):
                 step_converged()
             ms, launches = timed(step_converged, K, W)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, regime,
+                         dict(obs=sim.obs, reward=sim.reward, done=sim.done, a_prior=sim.a_prior, p=sim.p, dp=sim.dp,
+                              neighbor_index=sim.neighbor_index, in_flags=sim.in_flags, sensed_index=sim.sensed_index,
+                              occupied_index=sim.occupied_index), DUMP_BYTES // len(want))
         stats = all_reduce_stats(episode_stats(sim.reward, sim.in_flags)).tolist()   # episode statistics (not timed)
         regimes[regime] = {"ms_per_step": ms / K, "value": world * E * n_a * K / (ms * 1e-3), "gpu_launches": int(launches),
                            "roofline": roofline_of(ms / K, regime),

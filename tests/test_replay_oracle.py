@@ -1,13 +1,15 @@
-"""Pins oracle/replay_oracle.py to the reference's own ReplayBufferAgent (imported from /root/reference when present)."""
+"""Pins oracle/replay_oracle.py to the reference's own ReplayBufferAgent (imported from the checkout of the original project that
+oracle/live_reference.py locates, when present; tests/test_oracle_pins.py keeps the pin where it is not)."""
 import os
 import sys
 
 import numpy as np
 import pytest
 
+from oracle.live_reference import REF_ROOT
 from oracle.replay_oracle import ReplayOracle
 
-REF = "/root/reference/marl_llm/algorithm/utils"
+REF = os.path.join(REF_ROOT, "marl_llm", "algorithm", "utils")
 
 
 def _ref_class():
