@@ -330,6 +330,27 @@ int swarm_destroy(swarm_sim *s) {
     return SWARM_OK;
 }
 
+/* reads back which of envs [env0, env0 + count) matched a library shape (d_shape_id, written by the kernels that build grids) into
+ * the host mirror swarm_fast_path decides from; synchronises the stream */
+static int sync_shape_mirror(swarm_sim *s, int32_t env0, int32_t count, cudaStream_t st) {
+    std::vector<int> ids(count);
+    CU_TRY(cudaMemcpyAsync(ids.data(), s->d_shape_id + env0, sizeof(int) * count, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    for (int k = 0; k < count; ++k) {
+        const int old = s->h_shape_id[env0 + k];
+        s->n_unposed += (ids[k] < 0) - (old < 0);
+        s->n_inexact += (ids[k] < 0 || !(ids[k] & POSE_EXACT)) - (old < 0 || !(old & POSE_EXACT));
+        s->h_shape_id[env0 + k] = ids[k];
+    }
+    return SWARM_OK;
+}
+
+static bool every_shape_has_table(const swarm_sim *s) {
+    for (int k = 0; k < s->n_shapes; ++k)
+        if (!s->h_tabs[k].nb) return false;
+    return true;
+}
+
 int swarm_set_grid(swarm_sim *s, int32_t env0, int32_t count, const double *grid, int grid_on_device,
                    const int32_t *n_g, const double *l_cell, void *stream) {
     if (!s || !grid || !n_g || !l_cell) return fail(SWARM_ERR_INVALID, "null argument");
@@ -366,17 +387,10 @@ int swarm_set_grid(swarm_sim *s, int32_t env0, int32_t count, const double *grid
                                        s->buf.frame + (size_t)env0 * 2, A);
     CU_TRY(cudaGetLastError());
     s->launches++;
-    // which of these envs matched a library shape (lookup scan) — the host mirror decides which kernel a step launches
-    std::vector<int> ids(count);
-    CU_TRY(cudaMemcpyAsync(ids.data(), s->d_shape_id + env0, sizeof(int) * count, cudaMemcpyDeviceToHost, st));
-    // thr/n_g host vectors must outlive the async copies
-    CU_TRY(cudaStreamSynchronize(st));
-    for (int k = 0; k < count; ++k) {
-        const int old = s->h_shape_id[env0 + k];
-        s->n_unposed += (ids[k] < 0) - (old < 0);
-        s->n_inexact += (ids[k] < 0 || !(ids[k] & POSE_EXACT)) - (old < 0 || !(old & POSE_EXACT));
-        s->h_shape_id[env0 + k] = ids[k];
-    }
+    // which of these envs matched a library shape (lookup scan) — the host mirror decides which kernel a step launches.
+    // (its stream sync also keeps the thr/n_g host vectors alive until the async copies are done)
+    const int rc = sync_shape_mirror(s, env0, count, st);
+    if (rc != SWARM_OK) return rc;
     s->prior_dirty = true;
     return SWARM_OK;
 }
@@ -592,11 +606,15 @@ int swarm_reset(swarm_sim *s, uint64_t seed, uint64_t episode, uint64_t env_offs
     CU_TRY(cudaGetLastError());
     s->launches++;
     s->prior_dirty = true;
-    if (s->fast_ok && !env_mask) {
-        // every env now has a library pose (a shape without a table leaves its envs unmatched: rebuild the count)
-        bool all = true;
-        for (int k = 0; k < s->n_shapes; ++k) all = all && s->h_tabs[k].nb != 0;
-        if (all) { std::fill(s->h_shape_id.begin(), s->h_shape_id.end(), POSE_EXACT); s->n_unposed = 0; s->n_inexact = 0; }
+    if (s->fast_ok) {
+        if (!every_shape_has_table(s)) {
+            // an env that drew a shape without a table is unmatched now: the observe below must not run the lookup scan on it
+            const int rc = sync_shape_mirror(s, 0, s->cfg.num_envs, (cudaStream_t)stream);
+            if (rc != SWARM_OK) return rc;
+        } else if (!env_mask) {
+            // every env now has an exact library pose.  (A masked reset keeps the mirror: it only makes unmatched envs matched)
+            std::fill(s->h_shape_id.begin(), s->h_shape_id.end(), POSE_EXACT); s->n_unposed = 0; s->n_inexact = 0;
+        }
     }
     return swarm_observe(s, stream);     // ENV:221; a masked reset re-observes every env (idempotent for the untouched ones)
 }
@@ -618,12 +636,18 @@ int swarm_reset_envs(swarm_sim *s, uint64_t seed, uint64_t episode, uint64_t env
     R.in_thresh = s->buf.in_thresh; R.wbox = reinterpret_cast<float4 *>(s->buf.word_box); R.frame = s->buf.frame;
     R.nearest = s->buf.nearest_cell; R.info = info_dev; R.mask = nullptr; R.env_list = env_list_dev;
     R.seed = seed; R.episode = episode; R.env_offset = env_offset;
-    // (a partial reset keeps the host's matched-env count: matched envs stay matched; unmatched ones in the list become
-    // matched on the device but the host cannot tell which, so the general kernel stays in use until a full reset / set_grid)
     R.pose = s->fast_ok ? s->d_pose : nullptr; R.shape_id = s->fast_ok ? s->d_shape_id : nullptr; R.tabs = s->d_tabs;
     k_reset<<<count, 128, 0, (cudaStream_t)stream>>>(R);
     CU_TRY(cudaGetLastError());
     s->launches++;
+    // When every library shape has a table, the host keeps its matched-env count without a sync: matched envs stay matched;
+    // unmatched ones in the list become matched on the device, which the host does not track, so the general kernel stays in
+    // use until a full reset / set_grid.  Otherwise a listed env may have drawn a shape without a table and become unmatched:
+    // the mirror is read back before the observe below picks its kernel.
+    if (s->fast_ok && !every_shape_has_table(s)) {
+        const int rc = sync_shape_mirror(s, 0, s->cfg.num_envs, (cudaStream_t)stream);
+        if (rc != SWARM_OK) return rc;
+    }
     // observation + prior of the new state for the listed envs only; the others keep theirs (the a_prior buffer written is the
     // one holding the prior of the CURRENT state, which the next step returns)
     return launch_step(s, false, nullptr, SWARM_F32, (cudaStream_t)stream, env_list_dev, count);

@@ -21,6 +21,42 @@ def goal_seeking_action(obs, dp, rng, noise=0.3, target_row=28):
     return np.clip(a, -1, 1).astype(np.float32)
 
 
+def expected_grids(info, shapes):
+    """Grids of a device reset rebuilt from its draws (rows of reset_info): grid_center = R.origin + offset with the reference's
+    separately rounded products and sums (assembly.py:175-187)."""
+    grids = []
+    for row in info:
+        k, c, s, ox, oy = int(row[0]), row[1], row[2], row[3], row[4]
+        g = shapes["grid_origin"][k]
+        gx = (c * g[0] + s * g[1]) + ox
+        gy = ((-s) * g[0] + c * g[1]) + oy
+        grids.append(np.stack([gx, gy]))
+    return grids
+
+
+def oracle_follow_reset(ob, sim, shapes, rows, pick=None):
+    """After sim.reset / reset_envs: rebuild the oracle's envs `rows` from sim.reset_info (n_g, l_cell and grid from the shape
+    library `shapes`; p / dp from the simulator, whose values are the reference's map of the draws) and re-observe.  Oracle env k
+    is simulator env pick[k] (all envs in order without pick).  The oracle's observe must leave every other env's outputs as
+    they were: asserted."""
+    import torch
+    rows = np.asarray(rows, dtype=np.int64)
+    envs = rows if pick is None else np.asarray(pick)[rows]
+    te = torch.as_tensor(envs, device=sim.device)
+    info = sim.reset_info[te].cpu().numpy()
+    for k, row, g in zip(rows, info, expected_grids(info, shapes)):
+        ob.params[k].n_g = g.shape[1]
+        ob.params[k].l_cell = float(shapes["l_cell"][int(row[0])])
+        ob.set_grid(k, g)
+    ob.p[rows], ob.dp[rows] = sim.p[te].cpu().numpy(), sim.dp[te].cpu().numpy()
+    keep = np.setdiff1d(np.arange(ob.E), rows)
+    names = ("obs", "neighbor_index", "in_flags", "sensed_index", "occupied_index")
+    before = [getattr(ob, n)[keep].copy() for n in names]
+    ob.observe()
+    for n, b in zip(names, before):
+        assert np.array_equal(getattr(ob, n)[keep], b), f"oracle observe is not idempotent on {n}"
+
+
 def reset_like_reference(rng, n_a, shapes, half=2.4):
     """Domain randomisation in the spirit of assembly.py:156-223 (own RNG stream, not NumPy-global)."""
     k = int(rng.randint(0, len(shapes["l_cell"])))

@@ -8,7 +8,7 @@ import pytest
 import torch
 
 from oracle import oracle as orc
-from tests.helpers import goal_seeking_action, load_shapes
+from tests.helpers import expected_grids, goal_seeking_action, load_shapes
 
 pytestmark = pytest.mark.gpu
 
@@ -21,17 +21,6 @@ def make(E, n_a=30, **kw):
     sim = BatchedAssemblySim(E, n_a, ngm, r_avoid, out_dtype=torch.float64, emit_indices=True, **kw)
     sim.set_shapes(shapes["grid_origin"], shapes["l_cell"])
     return sim, shapes, r_avoid, ngm
-
-
-def expected_grids(info, shapes):
-    grids = []
-    for row in info:
-        k, c, s, ox, oy = int(row[0]), row[1], row[2], row[3], row[4]
-        g = shapes["grid_origin"][k]
-        gx = (c * g[0] + s * g[1]) + ox
-        gy = ((-s) * g[0] + c * g[1]) + oy
-        grids.append(np.stack([gx, gy]))
-    return grids
 
 
 def test_reset_state_is_the_reference_map_of_the_draws_and_rollout_matches_oracle():
