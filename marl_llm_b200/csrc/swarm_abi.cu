@@ -49,18 +49,12 @@ double thresh_le(double h) {
 
 int round32(int n) { return (n + 31) & ~31; }
 
-#ifdef SWARM_PH2_VEL_GLOBAL
-constexpr bool vel_global = true;
-#else
-constexpr bool vel_global = false;
-#endif
-size_t step_smem_bytes(int nt, int n_g_pad, int n_words, bool emit, int n_obs, int phase = 0, int rec_cap = -1, int lat_n = 0) {
-    (void)n_g_pad;
+size_t step_smem_bytes(int nt, int n_words, bool emit, int n_obs, int phase = 0, int rec_cap = -1, int lat_n = 0) {
     if (phase == 1)      // first half: state tile + 2 mbarrier slots (unused) + neighbour list + filter positions (k_step: SLIM)
         return (size_t)4 * nt * sizeof(double) + 16 + (size_t)TOPO * nt * sizeof(int) + (size_t)nt * sizeof(float2);
     size_t ring = (size_t)2 * CHUNK_CELLS * sizeof(double2);
     if (rec_cap >= 0) ring = std::max(ring, (size_t)(nt / 32) * ((size_t)4 * rec_cap + 128 + 16));      // lookup scan: per warp, row records + running counts
-    size_t b = ring + (rec_cap >= 0 ? 0 : (size_t)n_words * sizeof(float4)) + (size_t)(vel_global && phase == 2 ? 2 : 4) * nt * sizeof(double);   // TMA ring / records + word boxes + state tile
+    size_t b = ring + (rec_cap >= 0 ? 0 : (size_t)n_words * sizeof(float4)) + (size_t)4 * nt * sizeof(double);   // TMA ring / records + word boxes + state tile
     b += (size_t)n_words * nt * 4 * (emit ? 2 : 1);
     b += (size_t)((n_words + 3) & ~3) * 4 + 16;                                                    // covered mask + 2 mbarriers
     if (phase != 2) {                                                                                // the second-half kernel parks its neighbour list on the idle ring
@@ -88,44 +82,37 @@ cudaError_t raise_smem_limit(const void *fn, size_t bytes) {
     return e;
 }
 
-// phase 0 = the whole step in one launch; 1 / 2 = its two halves (single-warp envs)
-template <typename OUT, int MAXT, int PH>
-step_fn_t pick2(bool dyn, bool emit) {
-    if (dyn) return emit ? (step_fn_t)k_step<OUT, true, true, MAXT, PH> : (step_fn_t)k_step<OUT, true, false, MAXT, PH>;
-    return emit ? (step_fn_t)k_step<OUT, false, true, MAXT, PH> : (step_fn_t)k_step<OUT, false, false, MAXT, PH>;
+// grows a device staging buffer to hold at least n elements (its contents are not kept)
+template <typename T>
+int grow_staging(T *&buf, size_t &cap, size_t n) {
+    if (n <= cap) return SWARM_OK;
+    if (buf) CU_TRY(cudaFree(buf));
+    buf = nullptr; cap = 0;
+    CU_TRY(cudaMalloc(&buf, n * sizeof(T)));
+    cap = n;
+    return SWARM_OK;
 }
-// first half with a run-time block size (the flocking variant with more than 32 agents)
-step_fn_t pick_first_half_wide(bool f32, bool dyn) {
-    if (f32) return dyn ? (step_fn_t)k_step<float, true, false, 128, 1, 0, true> : (step_fn_t)k_step<float, false, false, 128, 1, 0, true>;
-    return dyn ? (step_fn_t)k_step<double, true, false, 128, 1, 0, true> : (step_fn_t)k_step<double, false, false, 128, 1, 0, true>;
+
+// The k_step instantiations the host launches, by key (template parameters: see k_step).  MAXT 1024 exists for PH 0 only and
+// WIDE for PH 1 only.  The first half never writes the index arrays, so it has no EMIT instantiation; the lookup-scan second
+// half (PH 2, FAST 1 / 2) exists for DYN = false only.
+template <typename OUT, bool DYN, bool EMIT>
+step_fn_t step_kernel(int maxt, int ph, int fast, bool wide) {
+    if (maxt == 1024)
+        return fast == 0 ? (step_fn_t)k_step<OUT, DYN, EMIT, 1024, 0>
+             : fast == 1 ? (step_fn_t)k_step<OUT, DYN, EMIT, 1024, 0, 1> : (step_fn_t)k_step<OUT, DYN, EMIT, 1024, 0, 2>;
+    if (ph == 0) return k_step<OUT, DYN, EMIT, 128, 0>;
+    if (ph == 1) return wide ? (step_fn_t)k_step<OUT, DYN, false, 128, 1, 0, true> : (step_fn_t)k_step<OUT, DYN, false, 128, 1>;
+    return fast == 0 ? (step_fn_t)k_step<OUT, DYN, EMIT, 128, 2>
+         : fast == 1 ? (step_fn_t)k_step<OUT, false, EMIT, 128, 2, 1> : (step_fn_t)k_step<OUT, false, EMIT, 128, 2, 2>;
 }
-// second half with the lookup scan (single-warp envs whose grids all have a known pose)
-// (exact: every pose is known exactly -> cells recomputed from the shape library instead of read per env)
-step_fn_t pick_fast(bool f32, bool emit, bool exact) {
-    if (exact) {
-        if (f32) return emit ? (step_fn_t)k_step<float, false, true, 128, 2, 2> : (step_fn_t)k_step<float, false, false, 128, 2, 2>;
-        return emit ? (step_fn_t)k_step<double, false, true, 128, 2, 2> : (step_fn_t)k_step<double, false, false, 128, 2, 2>;
+step_fn_t step_kernel(bool f32, bool dyn, bool emit, int maxt, int ph, int fast = 0, bool wide = false) {
+    if (f32) {
+        if (dyn) return emit ? step_kernel<float, true, true>(maxt, ph, fast, wide) : step_kernel<float, true, false>(maxt, ph, fast, wide);
+        return emit ? step_kernel<float, false, true>(maxt, ph, fast, wide) : step_kernel<float, false, false>(maxt, ph, fast, wide);
     }
-    if (f32) return emit ? (step_fn_t)k_step<float, false, true, 128, 2, 1> : (step_fn_t)k_step<float, false, false, 128, 2, 1>;
-    return emit ? (step_fn_t)k_step<double, false, true, 128, 2, 1> : (step_fn_t)k_step<double, false, false, 128, 2, 1>;
-}
-// multi-warp envs (more than 32 agents): the whole step in one launch, with the lookup scan
-template <typename OUT, int FASTV>
-step_fn_t pick_fast_big2(bool dyn, bool emit) {
-    if (dyn) return emit ? (step_fn_t)k_step<OUT, true, true, 1024, 0, FASTV> : (step_fn_t)k_step<OUT, true, false, 1024, 0, FASTV>;
-    return emit ? (step_fn_t)k_step<OUT, false, true, 1024, 0, FASTV> : (step_fn_t)k_step<OUT, false, false, 1024, 0, FASTV>;
-}
-step_fn_t pick_fast_big(bool f32, bool dyn, bool emit, bool exact) {
-    if (exact) return f32 ? pick_fast_big2<float, 2>(dyn, emit) : pick_fast_big2<double, 2>(dyn, emit);
-    return f32 ? pick_fast_big2<float, 1>(dyn, emit) : pick_fast_big2<double, 1>(dyn, emit);
-}
-step_fn_t pick_step(bool f32, bool dyn, bool emit, int nt, int phase = 0) {
-    if (nt <= 128) {
-        if (phase == 1) return f32 ? pick2<float, 128, 1>(dyn, emit) : pick2<double, 128, 1>(dyn, emit);
-        if (phase == 2) return f32 ? pick2<float, 128, 2>(false, emit) : pick2<double, 128, 2>(false, emit);
-        return f32 ? pick2<float, 128, 0>(dyn, emit) : pick2<double, 128, 0>(dyn, emit);
-    }
-    return f32 ? pick2<float, 1024, 0>(dyn, emit) : pick2<double, 1024, 0>(dyn, emit);
+    if (dyn) return emit ? step_kernel<double, true, true>(maxt, ph, fast, wide) : step_kernel<double, true, false>(maxt, ph, fast, wide);
+    return emit ? step_kernel<double, false, true>(maxt, ph, fast, wide) : step_kernel<double, false, false>(maxt, ph, fast, wide);
 }
 
 void fill_constants(KParams &K, int n_a, int n_g_max, int n_obs, int n_occ, bool self_state, bool want_prior,
@@ -162,6 +149,22 @@ void fill_constants(KParams &K, int n_a, int n_g_max, int n_obs, int n_occ, bool
 
 double in_shape_thresh(double l_cell) { return thresh_lt(std::sqrt(2.0) * l_cell / 2); }   // CPP:889
 
+// Host mirror of the per-env match record (d_shape_id) that swarm_fast_path decides from.  It must never call an env matched that
+// is not: the lookup kernel would index the table array with shape -1.  Every change goes through set(), which keeps the counts.
+struct MatchMirror {
+    enum State : unsigned char { UNMATCHED, DETECTED, EXACT };   // no library pose / pose detected (1e-9 accurate) / pose exact
+    std::vector<State> env;
+    long n_unposed = 0, n_inexact = 0;                           // envs UNMATCHED / not EXACT
+    void init(int n) { env.assign(n, UNMATCHED); n_unposed = n_inexact = n; }
+    void set(int e, State st) {
+        n_unposed += (st == UNMATCHED) - (env[e] == UNMATCHED);
+        n_inexact += (st != EXACT) - (env[e] != EXACT);
+        env[e] = st;
+    }
+    void set_all(State st) { for (int e = 0; e < (int)env.size(); ++e) set(e, st); }
+    static State of(int shape_id) { return shape_id < 0 ? UNMATCHED : (shape_id & POSE_EXACT) ? EXACT : DETECTED; }
+};
+
 }  // namespace
 
 struct swarm_sim {
@@ -171,7 +174,7 @@ struct swarm_sim {
     int nt;                 // threads per CTA
     bool split;             // step = two launches (k_step PH 1 + PH 2)
     size_t smem1;           // dynamic shared memory of the first half
-    size_t smem;            // dynamic shared memory of k_step PH 0 / 1
+    size_t smem;            // dynamic shared memory of k_step PH 0
     size_t smem2;           // ... of the second-half kernel (PH 2)
     int pending;            // a_prior buffer holding the prior of the CURRENT state
     int last;               // a_prior buffer returned by the most recent step
@@ -185,14 +188,31 @@ struct swarm_sim {
     // lookup scan: per-shape tables, per-env pose (library-owned device memory), host mirror of which envs are matched
     ShapeTab *d_tabs; std::vector<void *> tab_allocs; std::vector<ShapeTab> h_tabs;
     double4 *d_pose; int *d_shape_id;
-    std::vector<int> h_shape_id; long n_unposed, n_inexact;   // envs without a pose / with a pose that is only 1e-9 accurate
+    MatchMirror match;
     bool fast_ok;           // the shapes / sizes allow the lookup kernel at all
+    bool all_tables;        // every library shape has a table (a reset cannot leave an env unmatched)
     bool xy_exact;          // every library shape has bit-identical x per lattice column and y per lattice row
     int rec_cap; size_t smem_fast;
-    // chunked step: the two halves of a step are different kernels (issue bound / latency bound); chunks of the batch alternate
-    // between two internal streams so that the first half of one chunk overlaps the second half of another
-    cudaStream_t side[2]; cudaEvent_t ev_fork, ev_join[2]; int n_chunks;
 };
+
+// the k_step kernels launch_step runs for one step (dyn) or observe on a scan path (fast: see swarm_fast_path), and their dynamic
+// shared memory; k1 = nullptr when the step is one launch.  The shared-memory limits are raised for exactly these kernels.
+struct StepLaunch { step_fn_t k1, k2; size_t smem1, smem2; };
+static StepLaunch step_launch(const swarm_sim *s, bool dyn, int fast) {
+    const bool f32 = s->cfg.out_dtype == SWARM_F32, emit = s->cfg.emit_indices != 0;
+    const size_t smem_scan = fast ? s->smem_fast : s->split ? s->smem2 : s->smem;
+    // the second half runs no dynamics: observe and step share its DYN = false kernel
+    if (s->split) return {step_kernel(f32, dyn, emit, 128, 1), step_kernel(f32, false, emit, 128, 2, fast), s->smem1, smem_scan};
+    return {nullptr, step_kernel(f32, dyn, emit, (fast || s->nt > 128) ? 1024 : 128, 0, fast), 0, smem_scan};
+}
+static int raise_step_smem_limits(const swarm_sim *s, int fast) {
+    for (int dyn = 0; dyn < 2; ++dyn) {
+        const StepLaunch L = step_launch(s, dyn != 0, fast);
+        if (L.k1) CU_TRY(raise_smem_limit((const void *)L.k1, L.smem1));
+        CU_TRY(raise_smem_limit((const void *)L.k2, L.smem2));
+    }
+    return SWARM_OK;
+}
 
 extern "C" {
 
@@ -258,28 +278,21 @@ int swarm_create(const swarm_config *cfg, const swarm_buffers *buf, swarm_sim **
     K.nbr = buf->neighbor_index; K.in_flags = buf->in_flags; K.nearest = buf->nearest_cell;
     K.sensed = buf->sensed_index; K.occupied = buf->occupied_index;
     s->nt = round32(cfg->n_a);
-    s->smem = step_smem_bytes(s->nt, K.n_g_pad, K.n_words, cfg->emit_indices != 0, cfg->num_obs_grid_max);
-    s->smem2 = step_smem_bytes(s->nt, K.n_g_pad, K.n_words, cfg->emit_indices != 0, cfg->num_obs_grid_max, 2);
-    s->smem1 = step_smem_bytes(s->nt, K.n_g_pad, K.n_words, cfg->emit_indices != 0, cfg->num_obs_grid_max, 1);
-    if (const char *x = getenv("SWARM_DEBUG_EXTRA_SMEM")) s->smem += (size_t)atoi(x);   // occupancy experiments only
+    s->smem = step_smem_bytes(s->nt, K.n_words, cfg->emit_indices != 0, cfg->num_obs_grid_max);
+    s->smem2 = step_smem_bytes(s->nt, K.n_words, cfg->emit_indices != 0, cfg->num_obs_grid_max, 2);
+    s->smem1 = step_smem_bytes(s->nt, K.n_words, cfg->emit_indices != 0, cfg->num_obs_grid_max, 1);
     if (s->smem > (size_t)prop.sharedMemPerBlockOptin) {
         delete s;
         return fail(SWARM_ERR_UNSUPPORTED, "n_a x n_g_max needs more shared memory than one SM has");
     }
     s->split = (s->nt == 32) && !getenv("SWARM_FUSED_STEP");      // single-warp envs: two launches per step (see k_step, PH)
-    for (int dyn = 0; dyn < 2; ++dyn)
-        for (int ph = 0; ph < 3; ++ph) {
-            if (ph > 0 && s->nt > 128) continue;
-            step_fn_t f = pick_step(cfg->out_dtype == SWARM_F32, dyn != 0, cfg->emit_indices != 0, s->nt, ph);
-            cudaError_t e = raise_smem_limit((const void *)f, ph == 2 ? s->smem2 : s->smem);
-            if (e != cudaSuccess) { delete s; return fail(SWARM_ERR_CUDA, std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(e)); }
-        }
+    if (const int rc = raise_step_smem_limits(s, 0)) { delete s; return rc; }
     s->pending = 0; s->last = 0; s->prior_dirty = true; s->observed = false; s->launches = 0;
     s->d_stage = nullptr; s->stage_cap = 0; s->d_act = nullptr; s->act_cap = 0;
     s->d_shape_grid = nullptr; s->d_shape_ng = nullptr; s->d_shape_thr = nullptr; s->n_shapes = 0;
     s->d_tabs = nullptr; s->d_pose = nullptr; s->d_shape_id = nullptr;
-    s->h_shape_id.assign(cfg->num_envs, -1); s->n_unposed = cfg->num_envs; s->n_inexact = cfg->num_envs;
-    s->fast_ok = false; s->xy_exact = false; s->rec_cap = 0; s->smem_fast = 0;
+    s->match.init(cfg->num_envs);
+    s->fast_ok = false; s->all_tables = false; s->xy_exact = false; s->rec_cap = 0; s->smem_fast = 0;
     {
         cudaError_t e1 = cudaMalloc(&s->d_pose, sizeof(double4) * (size_t)cfg->num_envs);
         cudaError_t e2 = cudaMalloc(&s->d_shape_id, sizeof(int) * (size_t)cfg->num_envs);
@@ -292,22 +305,6 @@ int swarm_create(const swarm_config *cfg, const swarm_buffers *buf, swarm_sim **
         }
     }
     s->K.pose = s->d_pose; s->K.shape_id = s->d_shape_id;
-    s->side[0] = s->side[1] = nullptr; s->ev_fork = nullptr; s->ev_join[0] = s->ev_join[1] = nullptr;
-    s->n_chunks = 1;
-    if (s->split && cfg->num_envs >= 8192) {
-        // opt-in (SWARM_STEP_CHUNKS=2): measured 0.670 -> 0.663 ms per step with 2 chunks, 0.703 with 4, 0.817 with 8
-        // (profiles/r2_experiments.md) — not worth a fork/join on the caller's stream by default
-        int nc = 1;
-        if (const char *x = getenv("SWARM_STEP_CHUNKS")) nc = std::max(1, std::min(16, atoi(x)));
-        if (nc > 1) {
-            bool ok = cudaStreamCreateWithFlags(&s->side[0], cudaStreamNonBlocking) == cudaSuccess &&
-                      cudaStreamCreateWithFlags(&s->side[1], cudaStreamNonBlocking) == cudaSuccess &&
-                      cudaEventCreateWithFlags(&s->ev_fork, cudaEventDisableTiming) == cudaSuccess &&
-                      cudaEventCreateWithFlags(&s->ev_join[0], cudaEventDisableTiming) == cudaSuccess &&
-                      cudaEventCreateWithFlags(&s->ev_join[1], cudaEventDisableTiming) == cudaSuccess;
-            if (ok) s->n_chunks = nc; else cudaGetLastError();
-        }
-    }
     *out = s;
     return SWARM_OK;
 }
@@ -323,32 +320,19 @@ int swarm_destroy(swarm_sim *s) {
     if (s->d_pose) cudaFree(s->d_pose);
     if (s->d_shape_id) cudaFree(s->d_shape_id);
     if (s->d_tabs) cudaFree(s->d_tabs);
-    for (int k = 0; k < 2; ++k) { if (s->side[k]) cudaStreamDestroy(s->side[k]); if (s->ev_join[k]) cudaEventDestroy(s->ev_join[k]); }
-    if (s->ev_fork) cudaEventDestroy(s->ev_fork);
     for (void *q : s->tab_allocs) cudaFree(q);
     delete s;
     return SWARM_OK;
 }
 
 /* reads back which of envs [env0, env0 + count) matched a library shape (d_shape_id, written by the kernels that build grids) into
- * the host mirror swarm_fast_path decides from; synchronises the stream */
-static int sync_shape_mirror(swarm_sim *s, int32_t env0, int32_t count, cudaStream_t st) {
+ * the host mirror; synchronises the stream */
+static int sync_match(swarm_sim *s, int32_t env0, int32_t count, cudaStream_t st) {
     std::vector<int> ids(count);
     CU_TRY(cudaMemcpyAsync(ids.data(), s->d_shape_id + env0, sizeof(int) * count, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
-    for (int k = 0; k < count; ++k) {
-        const int old = s->h_shape_id[env0 + k];
-        s->n_unposed += (ids[k] < 0) - (old < 0);
-        s->n_inexact += (ids[k] < 0 || !(ids[k] & POSE_EXACT)) - (old < 0 || !(old & POSE_EXACT));
-        s->h_shape_id[env0 + k] = ids[k];
-    }
+    for (int k = 0; k < count; ++k) s->match.set(env0 + k, MatchMirror::of(ids[k]));
     return SWARM_OK;
-}
-
-static bool every_shape_has_table(const swarm_sim *s) {
-    for (int k = 0; k < s->n_shapes; ++k)
-        if (!s->h_tabs[k].nb) return false;
-    return true;
 }
 
 int swarm_set_grid(swarm_sim *s, int32_t env0, int32_t count, const double *grid, int grid_on_device,
@@ -368,12 +352,7 @@ int swarm_set_grid(swarm_sim *s, int32_t env0, int32_t count, const double *grid
     const double *src = grid;
     if (!grid_on_device) {
         const size_t need = (size_t)count * 2 * ngm;
-        if (need > s->stage_cap) {
-            if (s->d_stage) CU_TRY(cudaFree(s->d_stage));
-            s->d_stage = nullptr; s->stage_cap = 0;
-            CU_TRY(cudaMalloc(&s->d_stage, need * sizeof(double)));
-            s->stage_cap = need;
-        }
+        if (const int rc = grow_staging(s->d_stage, s->stage_cap, need)) return rc;
         CU_TRY(cudaMemcpyAsync(s->d_stage, grid, need * sizeof(double), cudaMemcpyHostToDevice, st));
         src = s->d_stage;
     }
@@ -389,8 +368,7 @@ int swarm_set_grid(swarm_sim *s, int32_t env0, int32_t count, const double *grid
     s->launches++;
     // which of these envs matched a library shape (lookup scan) — the host mirror decides which kernel a step launches.
     // (its stream sync also keeps the thr/n_g host vectors alive until the async copies are done)
-    const int rc = sync_shape_mirror(s, env0, count, st);
-    if (rc != SWARM_OK) return rc;
+    if (const int rc = sync_match(s, env0, count, st)) return rc;
     s->prior_dirty = true;
     return SWARM_OK;
 }
@@ -420,9 +398,8 @@ int swarm_set_shapes(swarm_sim *s, int32_t n_shapes, const double *grids, const 
     s->tab_allocs.clear();
     if (s->d_tabs) { cudaFree(s->d_tabs); s->d_tabs = nullptr; }
     CU_TRY(cudaMemset(s->d_shape_id, 0xFF, sizeof(int) * (size_t)s->cfg.num_envs));
-    std::fill(s->h_shape_id.begin(), s->h_shape_id.end(), -1);
-    s->n_unposed = s->cfg.num_envs; s->n_inexact = s->cfg.num_envs;
-    s->fast_ok = false; s->xy_exact = true;
+    s->match.set_all(MatchMirror::UNMATCHED);
+    s->fast_ok = false; s->all_tables = false; s->xy_exact = true;
     s->h_tabs.assign(n_shapes, ShapeTab{});
     // the lookup kernel serves single-warp envs with <= 1024 cells; rows per agent <= 32 and cells per row record <= 31
     double l_min = l_cell[0];
@@ -431,7 +408,7 @@ int swarm_set_shapes(swarm_sim *s, int32_t n_shapes, const double *grids, const 
     // (the lookup scan finds covered cells among an agent's sensing candidates: the covering radius must be the smaller one)
     const bool eligible = ((s->split && s->nt == 32) || (!s->split && s->nt > 32)) && s->K.n_words <= 32 && ngm <= 1023 && rr <= 14.9 && !s->cfg.brute_force_scan &&
                           0.5 * s->cfg.r_avoid + 1e-6 < s->cfg.d_sen &&
-                          !getenv("SWARM_NO_LOOKUP_SCAN") && !(s->nt > 32 && getenv("SWARM_NO_LOOKUP_SCAN_BIG"));
+                          !getenv("SWARM_NO_LOOKUP_SCAN");
     if (!eligible) return SWARM_OK;
     const double half_extent = std::max(s->K.half_w, s->K.half_h);
     // origin-frame positions the table must cover: |p| up to the walls (+ slack: they are soft), |offset| up to half - 1 (ENV:184-185)
@@ -504,6 +481,7 @@ int swarm_set_shapes(swarm_sim *s, int32_t n_shapes, const double *grids, const 
         ++n_tables;
     }
     CU_TRY(cudaDeviceSynchronize());
+    s->all_tables = n_tables == n_shapes;
     if (n_tables == 0) return SWARM_OK;
     // lattice blobs, all with lat_n entries per table (see ShapeTab::lattice)
     for (int k = 0; k < n_shapes; ++k) {
@@ -526,16 +504,12 @@ int swarm_set_shapes(swarm_sim *s, int32_t n_shapes, const double *grids, const 
     const int rows_per_agent = (2.0 * (rr + 2e-3) + 2.0 <= 16.0) ? 16 : 32;
     s->rec_cap = 32 * rows_per_agent;                              // per warp
     s->K.rec_cap = s->rec_cap;
-    const bool emit = s->cfg.emit_indices != 0, f32 = s->cfg.out_dtype == SWARM_F32;
-    s->smem_fast = step_smem_bytes(s->nt, s->K.n_g_pad, s->K.n_words, emit, s->cfg.num_obs_grid_max, s->split ? 2 : 0, s->rec_cap, lat_n);
-    if (const char *x = getenv("SWARM_DEBUG_EXTRA_SMEM_FAST")) s->smem_fast += (size_t)atoi(x);   // occupancy experiments only
+    s->smem_fast = step_smem_bytes(s->nt, s->K.n_words, s->cfg.emit_indices != 0, s->cfg.num_obs_grid_max, s->split ? 2 : 0, s->rec_cap, lat_n);
     cudaDeviceProp prop;
     CU_TRY(cudaGetDeviceProperties(&prop, s->cfg.device));
     if (s->smem_fast > (size_t)prop.sharedMemPerBlockOptin) return SWARM_OK;      // does not fit (e.g. 1024 agents with index arrays): general scan
-    for (int exact = 0; exact < 2; ++exact) {
-        if (s->split) CU_TRY(raise_smem_limit((const void *)pick_fast(f32, emit, exact != 0), s->smem_fast));
-        else for (int dyn = 0; dyn < 2; ++dyn) CU_TRY(raise_smem_limit((const void *)pick_fast_big(f32, dyn != 0, emit, exact != 0), s->smem_fast));
-    }
+    for (int fast = 1; fast <= 2; ++fast)
+        if (const int rc = raise_step_smem_limits(s, fast)) return rc;
     s->fast_ok = true;
     return SWARM_OK;
 }
@@ -552,12 +526,7 @@ int swarm_set_grid_pose(swarm_sim *s, int32_t env0, int32_t count, const int32_t
     cudaStream_t st = (cudaStream_t)stream;
     CU_TRY(cudaSetDevice(s->cfg.device));
     const size_t need = (size_t)count * 5;                       // staging: ids (as doubles' worth of space) + poses
-    if (need > s->stage_cap) {
-        if (s->d_stage) CU_TRY(cudaFree(s->d_stage));
-        s->d_stage = nullptr; s->stage_cap = 0;
-        CU_TRY(cudaMalloc(&s->d_stage, need * sizeof(double)));
-        s->stage_cap = need;
-    }
+    if (const int rc = grow_staging(s->d_stage, s->stage_cap, need)) return rc;
     double4 *d_pose_in = reinterpret_cast<double4 *>(s->d_stage);
     int *d_ids = reinterpret_cast<int *>(s->d_stage + (size_t)count * 4);
     CU_TRY(cudaMemcpyAsync(d_pose_in, pose, sizeof(double) * 4 * count, cudaMemcpyHostToDevice, st));
@@ -569,14 +538,7 @@ int swarm_set_grid_pose(swarm_sim *s, int32_t env0, int32_t count, const int32_t
                                             s->buf.frame + (size_t)env0 * 2, s->d_pose + env0, s->d_shape_id + env0);
     CU_TRY(cudaGetLastError());
     s->launches++;
-    CU_TRY(cudaStreamSynchronize(st));                           // the host arrays may go away
-    for (int k = 0; k < count; ++k) {
-        const int old = s->h_shape_id[env0 + k];
-        const int now = (s->fast_ok && s->h_tabs[shape_ids[k]].nb) ? (shape_ids[k] | POSE_EXACT) : -1;
-        s->n_unposed += (now < 0) - (old < 0);
-        s->n_inexact += (now < 0) - (old < 0 || !(old & POSE_EXACT));
-        s->h_shape_id[env0 + k] = now;
-    }
+    if (const int rc = sync_match(s, env0, count, st)) return rc;   // (its stream sync also lets the caller free the host arrays)
     s->prior_dirty = true;
     return SWARM_OK;
 }
@@ -584,8 +546,23 @@ int swarm_set_grid_pose(swarm_sim *s, int32_t env0, int32_t count, const int32_t
 /* which second-half kernel the next swarm_step / swarm_observe runs: 0 = general culled scan, 1 = lookup scan on the stored
  * cells (every env's grid matched a library shape), 2 = lookup scan with cells recomputed from the library (every pose exact) */
 int swarm_fast_path(const swarm_sim *s) {
-    if (!(s && s->fast_ok && s->n_unposed == 0)) return 0;
-    return (s->n_inexact == 0 && s->xy_exact && !getenv("SWARM_NO_EXACT_POSE")) ? 2 : 1;
+    if (!(s && s->fast_ok && s->match.n_unposed == 0)) return 0;
+    return (s->match.n_inexact == 0 && s->xy_exact) ? 2 : 1;
+}
+
+/* the k_reset arguments of swarm_reset / swarm_reset_envs: every env (env_mask and env_list NULL), the masked envs or the listed ones */
+static ResetParams reset_params(const swarm_sim *s, uint64_t seed, uint64_t episode, uint64_t env_offset, const uint8_t *env_mask,
+                                const int32_t *env_list, double *info_dev) {
+    ResetParams R;
+    R.n_a = s->cfg.n_a; R.n_g_pad = s->K.n_g_pad; R.n_g_cap = s->cfg.n_g_max; R.n_shapes = s->n_shapes;
+    R.half_w = s->K.half_w; R.half_h = s->K.half_h;
+    R.shape_grid = s->d_shape_grid; R.shape_n_g = s->d_shape_ng; R.shape_thresh = s->d_shape_thr;
+    R.p = s->buf.p; R.dp = s->buf.dp; R.grid = reinterpret_cast<double2 *>(s->buf.grid); R.n_g = s->buf.n_g;
+    R.in_thresh = s->buf.in_thresh; R.wbox = reinterpret_cast<float4 *>(s->buf.word_box); R.frame = s->buf.frame;
+    R.nearest = s->buf.nearest_cell; R.info = info_dev; R.mask = env_mask; R.env_list = env_list;
+    R.seed = seed; R.episode = episode; R.env_offset = env_offset;
+    R.pose = s->fast_ok ? s->d_pose : nullptr; R.shape_id = s->fast_ok ? s->d_shape_id : nullptr; R.tabs = s->d_tabs;
+    return R;
 }
 
 int swarm_reset(swarm_sim *s, uint64_t seed, uint64_t episode, uint64_t env_offset, const uint8_t *env_mask,
@@ -593,27 +570,17 @@ int swarm_reset(swarm_sim *s, uint64_t seed, uint64_t episode, uint64_t env_offs
     if (!s) return fail(SWARM_ERR_INVALID, "null handle");
     if (s->n_shapes <= 0) return fail(SWARM_ERR_INVALID, "swarm_reset before swarm_set_shapes");
     CU_TRY(cudaSetDevice(s->cfg.device));
-    ResetParams R;
-    R.n_a = s->cfg.n_a; R.n_g_pad = s->K.n_g_pad; R.n_g_cap = s->cfg.n_g_max; R.n_shapes = s->n_shapes;
-    R.half_w = s->K.half_w; R.half_h = s->K.half_h;
-    R.shape_grid = s->d_shape_grid; R.shape_n_g = s->d_shape_ng; R.shape_thresh = s->d_shape_thr;
-    R.p = s->buf.p; R.dp = s->buf.dp; R.grid = reinterpret_cast<double2 *>(s->buf.grid); R.n_g = s->buf.n_g;
-    R.in_thresh = s->buf.in_thresh; R.wbox = reinterpret_cast<float4 *>(s->buf.word_box); R.frame = s->buf.frame;
-    R.nearest = s->buf.nearest_cell; R.info = info_dev; R.mask = env_mask; R.env_list = nullptr;
-    R.seed = seed; R.episode = episode; R.env_offset = env_offset;
-    R.pose = s->fast_ok ? s->d_pose : nullptr; R.shape_id = s->fast_ok ? s->d_shape_id : nullptr; R.tabs = s->d_tabs;
-    k_reset<<<s->cfg.num_envs, 128, 0, (cudaStream_t)stream>>>(R);
+    k_reset<<<s->cfg.num_envs, 128, 0, (cudaStream_t)stream>>>(reset_params(s, seed, episode, env_offset, env_mask, nullptr, info_dev));
     CU_TRY(cudaGetLastError());
     s->launches++;
     s->prior_dirty = true;
     if (s->fast_ok) {
-        if (!every_shape_has_table(s)) {
+        if (!s->all_tables) {
             // an env that drew a shape without a table is unmatched now: the observe below must not run the lookup scan on it
-            const int rc = sync_shape_mirror(s, 0, s->cfg.num_envs, (cudaStream_t)stream);
-            if (rc != SWARM_OK) return rc;
+            if (const int rc = sync_match(s, 0, s->cfg.num_envs, (cudaStream_t)stream)) return rc;
         } else if (!env_mask) {
             // every env now has an exact library pose.  (A masked reset keeps the mirror: it only makes unmatched envs matched)
-            std::fill(s->h_shape_id.begin(), s->h_shape_id.end(), POSE_EXACT); s->n_unposed = 0; s->n_inexact = 0;
+            s->match.set_all(MatchMirror::EXACT);
         }
     }
     return swarm_observe(s, stream);     // ENV:221; a masked reset re-observes every env (idempotent for the untouched ones)
@@ -628,26 +595,15 @@ int swarm_reset_envs(swarm_sim *s, uint64_t seed, uint64_t episode, uint64_t env
     if (s->n_shapes <= 0) return fail(SWARM_ERR_INVALID, "swarm_reset_envs before swarm_set_shapes");
     if (!s->observed) return fail(SWARM_ERR_INVALID, "swarm_reset_envs needs a full reset / observe first");
     CU_TRY(cudaSetDevice(s->cfg.device));
-    ResetParams R;
-    R.n_a = s->cfg.n_a; R.n_g_pad = s->K.n_g_pad; R.n_g_cap = s->cfg.n_g_max; R.n_shapes = s->n_shapes;
-    R.half_w = s->K.half_w; R.half_h = s->K.half_h;
-    R.shape_grid = s->d_shape_grid; R.shape_n_g = s->d_shape_ng; R.shape_thresh = s->d_shape_thr;
-    R.p = s->buf.p; R.dp = s->buf.dp; R.grid = reinterpret_cast<double2 *>(s->buf.grid); R.n_g = s->buf.n_g;
-    R.in_thresh = s->buf.in_thresh; R.wbox = reinterpret_cast<float4 *>(s->buf.word_box); R.frame = s->buf.frame;
-    R.nearest = s->buf.nearest_cell; R.info = info_dev; R.mask = nullptr; R.env_list = env_list_dev;
-    R.seed = seed; R.episode = episode; R.env_offset = env_offset;
-    R.pose = s->fast_ok ? s->d_pose : nullptr; R.shape_id = s->fast_ok ? s->d_shape_id : nullptr; R.tabs = s->d_tabs;
-    k_reset<<<count, 128, 0, (cudaStream_t)stream>>>(R);
+    k_reset<<<count, 128, 0, (cudaStream_t)stream>>>(reset_params(s, seed, episode, env_offset, nullptr, env_list_dev, info_dev));
     CU_TRY(cudaGetLastError());
     s->launches++;
     // When every library shape has a table, the host keeps its matched-env count without a sync: matched envs stay matched;
     // unmatched ones in the list become matched on the device, which the host does not track, so the general kernel stays in
     // use until a full reset / set_grid.  Otherwise a listed env may have drawn a shape without a table and become unmatched:
     // the mirror is read back before the observe below picks its kernel.
-    if (s->fast_ok && !every_shape_has_table(s)) {
-        const int rc = sync_shape_mirror(s, 0, s->cfg.num_envs, (cudaStream_t)stream);
-        if (rc != SWARM_OK) return rc;
-    }
+    if (s->fast_ok && !s->all_tables)
+        if (const int rc = sync_match(s, 0, s->cfg.num_envs, (cudaStream_t)stream)) return rc;
     // observation + prior of the new state for the listed envs only; the others keep theirs (the a_prior buffer written is the
     // one holding the prior of the CURRENT state, which the next step returns)
     return launch_step(s, false, nullptr, SWARM_F32, (cudaStream_t)stream, env_list_dev, count);
@@ -758,37 +714,10 @@ static int launch_step(swarm_sim *s, bool dyn, const void *act, int act_dtype, c
     K.prior_next = s->buf.a_prior[dyn ? (1 - s->pending) : s->pending];
     K.env_list = env_list;
     const int ctas = env_list ? count : s->cfg.num_envs;
-    const bool f32 = s->cfg.out_dtype == SWARM_F32, emit = s->cfg.emit_indices != 0;
-    if (s->split) {
-        const int fp = swarm_fast_path(s);
-        step_fn_t k1 = pick_step(f32, dyn, emit, s->nt, 1);
-        step_fn_t k2 = fp ? pick_fast(f32, emit, fp == 2) : pick_step(f32, dyn, emit, s->nt, 2);
-        const size_t sm2 = fp ? s->smem_fast : s->smem2;
-        if (!env_list && s->n_chunks > 1) {
-            // fork: both side streams wait for the caller's stream; chunk c runs on side stream c % 2 (first half, then second
-            // half: same stream, so in order); join: the caller's stream waits for both
-            CU_TRY(cudaEventRecord(s->ev_fork, st));
-            for (int k = 0; k < 2; ++k) CU_TRY(cudaStreamWaitEvent(s->side[k], s->ev_fork, 0));
-            const int per = (ctas + s->n_chunks - 1) / s->n_chunks;
-            for (int c = 0; c < s->n_chunks; ++c) {
-                K.env0 = c * per;
-                const int n = std::min(per, ctas - K.env0);
-                if (n <= 0) break;
-                k1<<<n, s->nt, s->smem1, s->side[c & 1]>>>(K);
-                k2<<<n, s->nt, sm2, s->side[c & 1]>>>(K);
-                s->launches += 2;
-            }
-            for (int k = 0; k < 2; ++k) { CU_TRY(cudaEventRecord(s->ev_join[k], s->side[k])); CU_TRY(cudaStreamWaitEvent(st, s->ev_join[k], 0)); }
-        } else {
-            k1<<<ctas, s->nt, s->smem1, st>>>(K);
-            k2<<<ctas, s->nt, sm2, st>>>(K);
-            s->launches += 2;
-        }
-    } else {
-        if (const int fp = swarm_fast_path(s)) pick_fast_big(f32, dyn, emit, fp == 2)<<<ctas, s->nt, s->smem_fast, st>>>(K);
-        else pick_step(f32, dyn, emit, s->nt, 0)<<<ctas, s->nt, s->smem, st>>>(K);
-        s->launches++;
-    }
+    const StepLaunch L = step_launch(s, dyn, swarm_fast_path(s));
+    if (L.k1) { L.k1<<<ctas, s->nt, L.smem1, st>>>(K); s->launches++; }
+    L.k2<<<ctas, s->nt, L.smem2, st>>>(K);
+    s->launches++;
     CU_TRY(cudaGetLastError());
     return SWARM_OK;
 }
@@ -799,7 +728,8 @@ static int flock_launch(swarm_sim *s, bool dyn, const void *act, int act_dtype, 
     KParams K = s->K;
     K.act = act; K.act_f32 = (act_dtype == SWARM_F32);
     const bool f32 = s->cfg.out_dtype == SWARM_F32;
-    step_fn_t k1 = s->nt == 32 ? pick_step(f32, dyn, false, 32, 1) : pick_first_half_wide(f32, dyn);   // the assembly step's first half, unchanged
+    // the assembly step's first half, unchanged (its shared memory, 8 KB at most, needs no raised limit)
+    step_fn_t k1 = step_kernel(f32, dyn, false, 128, 1, 0, s->nt != 32);
     k1<<<s->cfg.num_envs, s->nt, s->smem1, st>>>(K);
     const double d_ref = 2.0 * s->cfg.r_avoid;
     if (f32) k_flock_reward<float><<<s->cfg.num_envs, s->nt, 0, st>>>(s->cfg.n_a, K.p, K.dp, K.nbr, K.T_avoid, d_ref, 1.0, 0.5, 0.5, K.periodic, K.half_w, K.half_h, (float *)s->buf.reward);
@@ -909,12 +839,7 @@ int swarm_step_host(swarm_sim *s, const float *act_host, void *obs_host, void *r
     CU_TRY(cudaSetDevice(s->cfg.device));
     const size_t E = s->cfg.num_envs, n = s->cfg.n_a;
     const size_t nact = E * 2 * n;
-    if (nact > s->act_cap) {
-        if (s->d_act) CU_TRY(cudaFree(s->d_act));
-        s->d_act = nullptr; s->act_cap = 0;
-        CU_TRY(cudaMalloc(&s->d_act, nact * sizeof(float)));
-        s->act_cap = nact;
-    }
+    if (const int rc = grow_staging(s->d_act, s->act_cap, nact)) return rc;
     CU_TRY(cudaMemcpyAsync(s->d_act, act_host, nact * sizeof(float), cudaMemcpyHostToDevice, st));
     int rc = swarm_step(s, s->d_act, SWARM_F32, stream);
     if (rc != SWARM_OK) return rc;
@@ -1085,7 +1010,7 @@ void _get_observation(double *p, double *dp, double *heading, double *obs, doubl
     if (K.obs_dim != obs_dim_agent) legacy_die(W, "obs_dim_agent does not match 2*2*(6+1+self)+2*num_obs_grid_max");
     K.E = 1;
     const int nt = round32(n_a);
-    const size_t smem = step_smem_bytes(nt, K.n_g_pad, K.n_words, true, num_obs_grid_max);
+    const size_t smem = step_smem_bytes(nt, K.n_words, true, num_obs_grid_max);
     const size_t n_obs = (size_t)K.obs_dim * n_a;
     legacy_grid(W, grid_center, n_g, l_cell);
     Xfer X(al(4 * (size_t)n_a * 8) * 2 + al(n_obs * 8) + al((size_t)n_a * 8 * 3) + al((size_t)n_a * TOPO * 4) + al((size_t)n_a * 8) +
@@ -1102,7 +1027,7 @@ void _get_observation(double *p, double *dp, double *heading, double *obs, doubl
     K.p = d_p; K.dp = d_dp; K.grid = g_grid.cells; K.n_g = g_grid.d_ng; K.in_thresh = g_grid.d_thr;
     K.obs = d_obs; K.reward = d_rew; K.prior_next = d_prior;
     K.nbr = d_nbr; K.in_flags = d_inf; K.nearest = d_near; K.sensed = d_sidx; K.occupied = d_occ;
-    step_fn_t f = pick_step(false, false, true, nt);
+    step_fn_t f = step_kernel(false, false, true, nt <= 128 ? 128 : 1024, 0);
     LEG_TRY(W, raise_smem_limit((const void *)f, smem));
     f<<<1, nt, smem>>>(K);
     LEG_TRY(W, cudaGetLastError());
