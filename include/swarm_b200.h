@@ -207,6 +207,50 @@ int swarm_selftest_division(int32_t device, uint64_t n, uint64_t seed, int32_t k
  * {coverage_rate, distribution_uniformity, voronoi_based_uniformity} (assembly_wrapper.py:48-72, 74-101, 103-129). */
 int swarm_metrics(swarm_sim *sim, double *out_dev, void *stream);
 
+/* ---- Rendering: rgb_array frames (gym's layout, uint8 [count][height][width][3]) of any set of envs, on the device.
+ * Pixel rules, all fp64 with every operation rounded separately (the library is built with -fmad=false):
+ *   view (x0, y1, x1, y0) = (xmin, ymax, xmax, ymin); sx = (x1 - x0) / W, sy = (y1 - y0) / H; the centre of pixel (row r, col c)
+ *   is X = x0 + (c + 0.5) * sx, Y = y1 - (r + 0.5) * sy (row 0 = top).  A disc (cx, cy, rr) covers it iff dx*dx + dy*dy <= rr,
+ *   dx = X - cx, dy = Y - cy, evaluated dx*dx, then dy*dy, then the sum.  Layers, bottom to top (the topmost covering one decides):
+ *   1. background: SWARM_RGB_ARENA if x_min <= X <= x_max && y_min <= Y <= y_max (the handle's boundary_pos), else SWARM_RGB_OUTSIDE;
+ *   2. SWARM_RENDER_CELLS: a disc at every cell j < n_g[e] with rr = in_thresh[e] * 0.5 (the in-shape radius), SWARM_RGB_CELL;
+ *   3. SWARM_RENDER_TRAILS: per agent a capsule around each segment A -> B of consecutive trail samples, half-width w = size_a * 0.25:
+ *      u = B - A, ll = ux*ux + uy*uy, t = ll > 0 ? ((X - Ax)*ux + (Y - Ay)*uy) / ll : 0 clamped to [0, 1], q = A + t*u, covered iff
+ *      (X - qx)^2 + (Y - qy)^2 <= w*w; a segment with |ux| > half_w or |uy| > half_h (a periodic wrap) is not drawn; SWARM_RGB_TRAIL;
+ *   4. SWARM_RENDER_AGENTS: a disc at p[e][:, i] with rr = size_a * size_a, SWARM_RGB_AGENT_IN if in_flags[e][i] & 1 (the last
+ *      observation) else SWARM_RGB_AGENT_OUT; where several agents cover a pixel the largest index wins.
+ * No anti-aliasing.  A flocking handle has no cells, and its agents all take SWARM_RGB_AGENT_OUT. */
+#define SWARM_RENDER_CELLS 1
+#define SWARM_RENDER_AGENTS 2
+#define SWARM_RENDER_TRAILS 4
+/* the palette, in this order (R, G, B) */
+#define SWARM_RGB_ARENA 255, 255, 255
+#define SWARM_RGB_OUTSIDE 160, 160, 160
+#define SWARM_RGB_CELL 190, 215, 240
+#define SWARM_RGB_TRAIL 250, 170, 90
+#define SWARM_RGB_AGENT_IN 40, 150, 40
+#define SWARM_RGB_AGENT_OUT 210, 40, 40
+typedef struct swarm_render_args {
+    int32_t struct_size;               /* sizeof(swarm_render_args)                                                    */
+    int32_t width, height;             /* pixels, each in [1, 8192]                                                      */
+    int32_t flags;                     /* SWARM_RENDER_* bits                                                            */
+    int32_t count;                     /* frames, >= 1                                                                   */
+    int32_t pad_;
+    const int32_t *env_ids;            /* HOST [count], each in [0, E); duplicates allowed                               */
+    double view[4];                    /* xmin, ymax, xmax, ymin (finite, xmin < xmax, ymin < ymax); all zero = the arena  */
+    const double *trail;               /* DEVICE ring [trail_cap][count][2][n_a] f64 of past positions, or NULL          */
+    int32_t trail_cap, trail_len;      /* 0 <= trail_len <= trail_cap <= 1024: the trail_len newest samples are drawn     */
+    int32_t trail_head;                /* ring slot of the newest sample, in [0, trail_cap) when trail_len > 0           */
+    int32_t pad2_;
+    uint8_t *frames;                   /* DEVICE [count][height][width][3]                                               */
+} swarm_render_args;
+/* Draws frame f of env env_ids[f] from the handle's current p, in_flags and cells.  Every argument is checked before anything is
+ * launched (SWARM_ERR_INVALID, frames untouched).  Stream-ordered, no host synchronisation; one launch per 2048 frames, counted in
+ * swarm_launch_count. */
+int swarm_render(swarm_sim *sim, const swarm_render_args *args, void *stream);
+/* Copies the palette (6 RGB triples in the order of the SWARM_RGB_* macros above) to rgb[18] unless NULL; returns 6. */
+int swarm_render_palette(uint8_t *rgb);
+
 /* The reference env's own action strategies (ENV:519-601, Python/NumPy there) for the CURRENT state of every env:
  * SWARM_STRATEGY_RULE = agent_strategy 'rule' (ENV:530-601, the expert controller of collect_expert_data.py),
  * SWARM_STRATEGY_LLM = 'llm' (ENV:524-529 -> robot_prior_policy ENV:876-941; uses the neighbour list of the last

@@ -39,6 +39,17 @@ class SwarmBuffers(C.Structure):
     ]
 
 
+SWARM_RENDER_CELLS, SWARM_RENDER_AGENTS, SWARM_RENDER_TRAILS = 1, 2, 4
+
+
+class SwarmRenderArgs(C.Structure):        # swarm_render_args
+    _fields_ = [
+        ("struct_size", C.c_int32), ("width", C.c_int32), ("height", C.c_int32), ("flags", C.c_int32), ("count", C.c_int32),
+        ("pad_", C.c_int32), ("env_ids", C.c_void_p), ("view", C.c_double * 4), ("trail", C.c_void_p), ("trail_cap", C.c_int32),
+        ("trail_len", C.c_int32), ("trail_head", C.c_int32), ("pad2_", C.c_int32), ("frames", C.c_void_p),
+    ]
+
+
 SWARM_PP_INPUT, SWARM_PP_STATIC, SWARM_PP_RANDOM, SWARM_PP_NEAREST = 0, 1, 2, 3
 
 
@@ -64,7 +75,8 @@ BATCHED_SYMBOLS = ["swarm_grid_pad", "swarm_obs_dim", "swarm_create", "swarm_des
                    "swarm_set_shapes", "swarm_reset", "swarm_metrics", "swarm_set_obs_buffer", "swarm_strategy_actions",
                    "swarm_mark_state_dirty", "swarm_observe", "swarm_step", "swarm_step_host", "swarm_a_prior_ptr",
                    "swarm_fill_actions", "swarm_launch_count", "swarm_kernel_geometry", "swarm_last_error",
-                   "swarm_abi_version", "swarm_sqrt_threshold", "swarm_debug_rho", "swarm_restore_observation", "swarm_is_observed", "swarm_reset_envs", "swarm_measure_fma_peak", "swarm_fast_path", "swarm_set_grid_pose", "swarm_flock_observe", "swarm_flock_step", "swarm_selftest_division", "swarm_pp_obs_dim", "swarm_pp_observe", "swarm_pp_step"]
+                   "swarm_abi_version", "swarm_sqrt_threshold", "swarm_debug_rho", "swarm_restore_observation", "swarm_is_observed", "swarm_reset_envs", "swarm_measure_fma_peak", "swarm_fast_path", "swarm_set_grid_pose", "swarm_flock_observe", "swarm_flock_step", "swarm_selftest_division", "swarm_pp_obs_dim", "swarm_pp_observe", "swarm_pp_step",
+                   "swarm_render", "swarm_render_palette"]
 ROLLOUT_SYMBOLS = ["swarm_rollout_push", "swarm_rollout_gather", "swarm_rollout_push_parts", "swarm_rollout_gather_ring"]
 SWARM_PUSH_OBS, SWARM_PUSH_NEXT_OBS, SWARM_PUSH_SMALL = 1, 2, 4
 POLICY_SYMBOLS = ["swarm_policy_create", "swarm_policy_destroy", "swarm_policy_load", "swarm_policy_step", "swarm_policy_launch_count",
@@ -114,6 +126,8 @@ def load():
     lib.swarm_set_obs_buffer.argtypes = [C.c_void_p, C.c_void_p]
     lib.swarm_strategy_actions.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
     lib.swarm_metrics.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.swarm_render.argtypes = [C.c_void_p, C.POINTER(SwarmRenderArgs), C.c_void_p]
+    lib.swarm_render_palette.argtypes = [C.c_void_p]
     lib.swarm_set_shapes.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.swarm_reset.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.swarm_reset_envs.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]

@@ -10,7 +10,8 @@ so that marl_llm/train/train_assembly.py and eval/eval_assembly.py see the env t
     env.p, env.dp, env.env.grid_center = ...            # readable and writable (eval_assembly.py:34-57,137-151)
 
 `num_envs > 1` gives a vectorised variant with a leading batch axis on every array (not in the reference).
-All arithmetic runs in the sm_100a kernels (marl_llm_b200/csrc); there is no CPU fallback.  render() is a no-op.
+All arithmetic runs in the sm_100a kernels (marl_llm_b200/csrc); there is no CPU fallback.  render("rgb_array") returns frames
+drawn on the device (marl_llm_b200/render.py); render() in "human" mode draws nothing and returns None.
 """
 import pickle
 
@@ -18,6 +19,9 @@ import numpy as np
 import torch
 
 from .batched import BatchedAssemblySim
+from .render import SwarmRenderer
+
+RGB_ARRAY_SIZE = 480        # render("rgb_array") frames are RGB_ARRAY_SIZE x RGB_ARRAY_SIZE pixels of the arena
 
 
 class Box:
@@ -49,6 +53,8 @@ class AssemblySwarmEnv:
         self.k_ball, self.k_wall, self.c_wall = 30, 100, 5
         self.simulation_time, self.dt, self.n_frames, self.sensitivity = 0, 0.1, 1, 1
         self._sim = None
+        self._rend = None
+        self.render_traj, self.traj_len = False, 15
         self._grid_dirty = False
         self.unwrapped = self
 
@@ -254,6 +260,9 @@ class AssemblySwarmEnv:
         self.ddp = np.zeros((2, self.n_a))
         self.heading = np.zeros((self.dim, self.n_a))
         self._sim.observe()
+        if self.render_traj:
+            self._renderer().clear()
+            self._renderer().record()
         return self.obs
 
     # ---------------------------------------------------------------------------------------- ENV:487-666
@@ -274,20 +283,42 @@ class AssemblySwarmEnv:
                 a = a.astype(np.float64)
             act = torch.from_numpy(a).reshape(self.num_envs, 2, self.n_a).to(self._sim.device)
         obs, rew, done, _, prior = self._sim.step(act)
+        if self.render_traj:
+            self._renderer().record()
         info = np.array([None, None, None]).reshape(3, 1)               # ENV:484-485
         u = a.astype(np.float64)
         last = u if self.is_collected else (self._host(prior) if prior is not None else None)   # ENV:663-666
         return self._host(obs), self._host(rew), self._host(done), info, last
 
+    def _renderer(self):
+        """The renderer of every env of the current handle (rebuilt with the handle, keeping the recorded trail)."""
+        r = self._rend
+        if r is None or r.sim is not self._sim:
+            new = SwarmRenderer(self._sim, np.arange(self.num_envs), RGB_ARRAY_SIZE, RGB_ARRAY_SIZE,
+                                trail_len=self.traj_len if self.render_traj else 0)
+            if r is not None and r.trail is not None and new.trail is not None:
+                new.trail.copy_(r.trail)
+                new.trail_len, new.trail_head = r.trail_len, r.trail_head
+            self._rend = r = new
+        return r
+
     def render(self, mode="human"):
-        """ENV:668-747 draws the swarm with matplotlib; drawing is outside the step() hot path, so this is a no-op that keeps
-        train_assembly.py:93-94 and eval_assembly.py:147 running unchanged (they ignore the return value)."""
-        return None
+        """ENV:668-747 draws the swarm with matplotlib.  mode="rgb_array": a uint8 [480, 480, 3] frame of the arena drawn on the
+        device ([E, 480, 480, 3] with num_envs > 1): the env's target cells, the trails of the last traj_len positions when
+        render_traj is set, and the agents, green inside the shape and red outside (DESIGN.md §10).  This draws the env's actual,
+        rotated cells, where the reference shows the un-rotated source bitmap at shape_bound_points.  Any other mode draws
+        nothing and returns None, which keeps train_assembly.py:93-94 and eval_assembly.py:147 unchanged."""
+        if mode != "rgb_array":
+            return None
+        if self._grid_dirty:
+            self._push_grid()
+        return self._host(self._renderer().render())
 
     def close(self):
         if self._sim is not None:
             self._sim.close()
             self._sim = None
+        self._rend = None
 
 
 class Agent:

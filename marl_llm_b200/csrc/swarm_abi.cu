@@ -3,6 +3,7 @@
 // There is no CPU implementation behind these entry points: without a usable sm_100 device the batched calls
 // return SWARM_ERR_NO_DEVICE / SWARM_ERR_CUDA and the legacy (void) calls print the CUDA error and abort.
 #include "swarm_kernels.cuh"
+#include "render_kernels.cuh"
 #include "../../include/swarm_b200.h"
 
 #include <algorithm>
@@ -666,6 +667,66 @@ int swarm_metrics(swarm_sim *s, double *out_dev, void *stream) {
                                                                     thresh_lt(s->cfg.r_avoid / 2), out_dev);
     CU_TRY(cudaGetLastError());
     s->launches++;
+    return SWARM_OK;
+}
+
+int swarm_render_palette(uint8_t *rgb) {
+    static const uint8_t pal[RC_COUNT * 3] = {SWARM_RGB_ARENA, SWARM_RGB_OUTSIDE, SWARM_RGB_CELL, SWARM_RGB_TRAIL,
+                                              SWARM_RGB_AGENT_IN, SWARM_RGB_AGENT_OUT};
+    if (rgb) memcpy(rgb, pal, sizeof(pal));
+    return RC_COUNT;
+}
+
+int swarm_render(swarm_sim *s, const swarm_render_args *a, void *stream) {
+    if (!s || !a) return fail(SWARM_ERR_INVALID, "null argument");
+    if (a->struct_size != (int32_t)sizeof(swarm_render_args)) return fail(SWARM_ERR_INVALID, "struct_size mismatch (ABI)");
+    if (a->width < 1 || a->width > 8192 || a->height < 1 || a->height > 8192)
+        return fail(SWARM_ERR_INVALID, "width and height must be in [1, 8192]");
+    if (a->flags & ~(SWARM_RENDER_CELLS | SWARM_RENDER_AGENTS | SWARM_RENDER_TRAILS)) return fail(SWARM_ERR_INVALID, "unknown flags");
+    if (a->count < 1 || !a->env_ids) return fail(SWARM_ERR_INVALID, "count must be >= 1 with a non-NULL env_ids");
+    for (int f = 0; f < a->count; ++f)
+        if (a->env_ids[f] < 0 || a->env_ids[f] >= s->cfg.num_envs) return fail(SWARM_ERR_INVALID, "env id out of range");
+    const double *bp = s->cfg.boundary_pos;
+    const bool arena = a->view[0] == 0 && a->view[1] == 0 && a->view[2] == 0 && a->view[3] == 0;
+    const double *v = arena ? bp : a->view;
+    const double sx = (v[2] - v[0]) / a->width, sy = (v[1] - v[3]) / a->height;
+    for (int k = 0; k < 4; ++k)
+        if (!std::isfinite(v[k])) return fail(SWARM_ERR_INVALID, "view must be finite");
+    if (!(v[0] < v[2] && v[3] < v[1]) || !std::isfinite(sx) || !std::isfinite(sy) || !(sx > 0) || !(sy > 0))
+        return fail(SWARM_ERR_INVALID, "view needs xmin < xmax and ymin < ymax");
+    if (a->trail_len < 0 || a->trail_len > a->trail_cap || a->trail_cap > 1024)
+        return fail(SWARM_ERR_INVALID, "trail: 0 <= trail_len <= trail_cap <= 1024");
+    if (a->trail_len > 0 && (!a->trail || a->trail_head < 0 || a->trail_head >= a->trail_cap))
+        return fail(SWARM_ERR_INVALID, "trail: a non-NULL ring and 0 <= trail_head < trail_cap");
+    if (!a->frames) return fail(SWARM_ERR_INVALID, "frames is NULL");
+    CU_TRY(cudaSetDevice(s->cfg.device));
+
+    RenderParams P{};
+    const double size_a = s->cfg.size_a;
+    P.W = a->width; P.H = a->height; P.flags = a->flags; P.n_a = s->cfg.n_a; P.n_g_pad = s->K.n_g_pad; P.count = a->count;
+    P.cells_ok = s->cfg.variant == SWARM_VARIANT_ASSEMBLY;
+    P.trail_cap = a->trail_cap; P.trail_len = a->trail_len; P.trail_head = a->trail_head;
+    P.x0 = v[0]; P.y1 = v[1]; P.sx = sx; P.sy = sy;
+    // cull margin: one pixel, plus slack for the roundings of the (inexact) box tests
+    const double slack = 1e-12 * (std::fabs(v[0]) + std::fabs(v[1]) + std::fabs(v[2]) + std::fabs(v[3]) + 1.0);
+    P.mx = sx + slack; P.my = sy + slack;
+    P.ax0 = bp[0]; P.ay1 = bp[1]; P.ax1 = bp[2]; P.ay0 = bp[3];
+    P.rr_agent = size_a * size_a; P.r_agent = size_a;
+    P.w = size_a * 0.25; P.ww = P.w * P.w;
+    P.half_w = s->K.half_w; P.half_h = s->K.half_h;
+    P.p = s->buf.p; P.in_flags = s->buf.in_flags; P.grid = reinterpret_cast<const double2 *>(s->buf.grid);
+    P.n_g = s->buf.n_g; P.in_thresh = s->buf.in_thresh;
+    P.trail = a->trail; P.frames = a->frames;
+    swarm_render_palette(&P.palette[0][0]);
+    const dim3 tiles((a->width + RENDER_TILE - 1) / RENDER_TILE, (a->height + RENDER_TILE - 1) / RENDER_TILE);
+    for (int f0 = 0; f0 < a->count; f0 += RENDER_IDS_PER_LAUNCH) {
+        const int n = std::min(a->count - f0, RENDER_IDS_PER_LAUNCH);
+        P.f0 = f0;
+        memcpy(P.env, a->env_ids + f0, sizeof(int32_t) * n);
+        k_render<<<dim3(tiles.x, tiles.y, n), RENDER_THREADS, 0, (cudaStream_t)stream>>>(P);
+        CU_TRY(cudaGetLastError());
+        s->launches++;
+    }
     return SWARM_OK;
 }
 
