@@ -19,6 +19,22 @@ int pfail(int code, const std::string &m) { return swarm_set_last_error_(code, m
         if (err__ != cudaSuccess) return pfail(SWARM_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(err__)); \
     } while (0)
 constexpr size_t POL_SMEM = ((size_t)2 * POL_HP * POL_M + (size_t)2 * POL_KC * POL_HP) * sizeof(float);
+
+// the kernel swarm_policy_step launches for a precision (SWARM_POLICY_*) and rows_out on or off, with its block size and
+// its dynamic shared memory for act_dim A (the FFMA kernel writes rows_out without a template switch)
+struct PolicyKernel { const void *fn; int threads; size_t smem; };
+PolicyKernel policy_kernel(int precision, bool rows, int A) {
+    static const void *const fn[3][2] = {
+        {(const void *)k_policy_mlp, (const void *)k_policy_mlp},
+        {(const void *)k_policy_mlp_tc<false>, (const void *)k_policy_mlp_tc<true>},
+        {(const void *)k_policy_mlp_tc3<false>, (const void *)k_policy_mlp_tc3<true>}};
+    static const int threads[3] = {POL_THREADS, TC_THREADS, T3_THREADS};
+    return {fn[precision][rows], threads[precision], precision == SWARM_POLICY_FP32 ? POL_SMEM : tc_smem_bytes(A)};
+}
+
+// byte offset of W[n][k] in one layer of the tensor-core paths' weights: the canonical K-major no-swizzle UMMA layout,
+// 8-row x 16-byte core matrices
+size_t umma_byte(int k, int n) { return (size_t)(k / 8) * TC_LBO + (size_t)(n / 8) * TC_SBO + (size_t)(n % 8) * 16 + (size_t)(k % 8) * 2; }
 }  // namespace
 
 struct swarm_policy {
@@ -26,7 +42,7 @@ struct swarm_policy {
     float *d_w;          // one allocation: Wt[3][HP][HP], b[3][HP], W4[A][HP], b4[A]
     unsigned char *d_w16; // [3][TC_W_BYTES] fp16 weights in the canonical UMMA K-major layout (tensor-core path)
     unsigned char *d_w16x; // [6][TC_W_BYTES] hi/lo fp16 split of the weights, chunk order H1 L1 H2 L2 H3 L3 (fp32-accurate tensor-core path)
-    int precision;       // SWARM_POLICY_FP32 | SWARM_POLICY_F16_TC
+    int precision;       // SWARM_POLICY_FP32 | SWARM_POLICY_F16_TC | SWARM_POLICY_F16X3_TC
     int n_sm;
     float *debug;        // test hook: layer-1 accumulators of the tensor-core path
     float *rows_out;     // optional agent-major copy of the observations (swarm_policy_rows_out)
@@ -60,11 +76,11 @@ int swarm_policy_create(int32_t device, int32_t obs_dim, int32_t hidden_dim, int
     if (e != cudaSuccess) { delete p; return pfail(SWARM_ERR_CUDA, std::string("cudaMalloc: ") + cudaGetErrorString(e)); }
     if (e == cudaSuccess) e = cudaMalloc(&p->d_w16, (size_t)3 * TC_W_BYTES);
     if (e == cudaSuccess) e = cudaMalloc(&p->d_w16x, (size_t)6 * TC_W_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute((const void *)k_policy_mlp_tc3<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(TC_AMAX));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute((const void *)k_policy_mlp_tc3<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(TC_AMAX));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute((const void *)k_policy_mlp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)POL_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute((const void *)k_policy_mlp_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(TC_AMAX));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute((const void *)k_policy_mlp_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(TC_AMAX));
+    for (int prec : {SWARM_POLICY_FP32, SWARM_POLICY_F16_TC, SWARM_POLICY_F16X3_TC})
+        for (bool rows : {false, true}) {
+            const PolicyKernel k = policy_kernel(prec, rows, TC_AMAX);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem);
+        }
     if (e != cudaSuccess) { cudaFree(p->d_w); cudaFree(p->d_w16); cudaFree(p->d_w16x); delete p; return pfail(SWARM_ERR_CUDA, std::string("policy setup: ") + cudaGetErrorString(e)); }
     *out = p;
     return SWARM_OK;
@@ -87,12 +103,27 @@ int swarm_policy_load(swarm_policy *p, const float *w1, const float *b1, const f
     const int H = p->hidden, K0 = p->obs_dim, A = p->act_dim;
     const size_t n = (size_t)3 * POL_HP * POL_HP + 3 * POL_HP + (size_t)A * POL_HP + A;
     std::vector<float> h(n, 0.f);
+    // every weight W[n][k] (torch Linear.weight is [out][in]) goes to three copies, all zero-padded to 192 x 192:
+    //   fp32 path: Wt[k][n];
+    //   tensor-core path: fp16 in the UMMA layout (umma_byte);
+    //   fp32-accurate tensor-core path: w = hi + lo with hi = fp16(w), lo = fp16(w - hi), same layout, chunks H1 L1 H2 L2 H3 L3
+    std::vector<__half> h16((size_t)3 * POL_HP * POL_HP, __float2half(0.f));
+    std::vector<__half> hx((size_t)6 * POL_HP * POL_HP, __float2half(0.f));
     const float *W[3] = {w1, w2, w3}, *B[3] = {b1, b2, b3};
     const int Kin[3] = {K0, H, H};
     for (int l = 0; l < 3; ++l) {
-        float *wt = h.data() + (size_t)l * POL_HP * POL_HP;                       // Wt[k][n] = W[n][k] (torch Linear.weight is [out][in])
+        float *wt = h.data() + (size_t)l * POL_HP * POL_HP;
         for (int nn = 0; nn < H; ++nn)
-            for (int k = 0; k < Kin[l]; ++k) wt[(size_t)k * POL_HP + nn] = W[l][(size_t)nn * Kin[l] + k];
+            for (int k = 0; k < Kin[l]; ++k) {
+                const float w = W[l][(size_t)nn * Kin[l] + k];
+                const size_t u = umma_byte(k, nn) / 2;
+                wt[(size_t)k * POL_HP + nn] = w;
+                h16[(size_t)l * POL_HP * POL_HP + u] = __float2half_rn(w);
+                const float wc = w > 65504.f ? 65504.f : (w < -65504.f ? -65504.f : w);
+                const __half hi = __float2half_rn(wc);
+                hx[(size_t)(2 * l) * POL_HP * POL_HP + u] = hi;
+                hx[(size_t)(2 * l + 1) * POL_HP * POL_HP + u] = __float2half_rn(wc - __half2float(hi));
+            }
         float *bb = h.data() + (size_t)3 * POL_HP * POL_HP + (size_t)l * POL_HP;
         for (int nn = 0; nn < H; ++nn) bb[nn] = B[l][nn];
     }
@@ -101,29 +132,7 @@ int swarm_policy_load(swarm_policy *p, const float *w1, const float *b1, const f
         for (int k = 0; k < H; ++k) w4p[(size_t)j * POL_HP + k] = w4[(size_t)j * H + k];
     for (int j = 0; j < A; ++j) w4p[(size_t)A * POL_HP + j] = b4[j];
     PCU_TRY(cudaMemcpy(p->d_w, h.data(), n * sizeof(float), cudaMemcpyHostToDevice));
-    // tensor-core path: W[n][k] as fp16 in the canonical K-major no-swizzle UMMA layout: 8-row x 16-byte core matrices,
-    // byte address = (k/8) * TC_LBO + (n/8) * TC_SBO + (n%8) * 16 + (k%8) * 2; zero padding up to 192 x 192
-    std::vector<__half> h16((size_t)3 * POL_HP * POL_HP, __float2half(0.f));
-    for (int l = 0; l < 3; ++l)
-        for (int nn = 0; nn < H; ++nn)
-            for (int k = 0; k < Kin[l]; ++k) {
-                const size_t byte = (size_t)(k / 8) * TC_LBO + (size_t)(nn / 8) * TC_SBO + (size_t)(nn % 8) * 16 + (size_t)(k % 8) * 2;
-                h16[(size_t)l * POL_HP * POL_HP + byte / 2] = __float2half_rn(W[l][(size_t)nn * Kin[l] + k]);
-            }
     PCU_TRY(cudaMemcpy(p->d_w16, h16.data(), (size_t)3 * TC_W_BYTES, cudaMemcpyHostToDevice));
-    // fp32-accurate tensor-core path: w = hi + lo with hi = fp16(w), lo = fp16(w - hi); same layout, chunks H1 L1 H2 L2 H3 L3
-    std::vector<__half> hx((size_t)6 * POL_HP * POL_HP, __float2half(0.f));
-    for (int l = 0; l < 3; ++l)
-        for (int nn = 0; nn < H; ++nn)
-            for (int k = 0; k < Kin[l]; ++k) {
-                const size_t byte = (size_t)(k / 8) * TC_LBO + (size_t)(nn / 8) * TC_SBO + (size_t)(nn % 8) * 16 + (size_t)(k % 8) * 2;
-                float w = W[l][(size_t)nn * Kin[l] + k];
-                w = w > 65504.f ? 65504.f : (w < -65504.f ? -65504.f : w);
-                const __half hi = __float2half_rn(w);
-                const __half lo = __float2half_rn(w - __half2float(hi));
-                hx[(size_t)(2 * l) * POL_HP * POL_HP + byte / 2] = hi;
-                hx[(size_t)(2 * l + 1) * POL_HP * POL_HP + byte / 2] = lo;
-            }
     PCU_TRY(cudaMemcpy(p->d_w16x, hx.data(), (size_t)6 * TC_W_BYTES, cudaMemcpyHostToDevice));
     p->loaded = true;
     return SWARM_OK;
@@ -145,31 +154,19 @@ int swarm_policy_step(swarm_policy *p, const float *obs, int32_t num_envs, int32
     P.W4 = p->d_w + (size_t)3 * POL_HP * POL_HP + 3 * POL_HP;
     P.b4 = P.W4 + (size_t)p->act_dim * POL_HP;
     P.slope = 0.01f; P.explore = explore; P.scale = noise_scale; P.seed = seed; P.step = step;
-    if (p->precision == SWARM_POLICY_F16X3_TC) {
-        PolicyTcParams Q;
-        Q.base = P; Q.w16 = p->d_w16x; Q.small = p->d_w + (size_t)3 * POL_HP * POL_HP; Q.debug = p->debug;
+    const PolicyKernel k = policy_kernel(p->precision, p->rows_out != nullptr, p->act_dim);
+    PolicyTcParams Q;
+    void *args[1] = {&P};
+    unsigned grid = (unsigned)((P.n_cols + POL_M - 1) / POL_M);
+    if (p->precision != SWARM_POLICY_FP32) {
+        Q.base = P; Q.w16 = p->precision == SWARM_POLICY_F16_TC ? p->d_w16 : p->d_w16x;
+        Q.small = p->d_w + (size_t)3 * POL_HP * POL_HP; Q.debug = p->debug;
         Q.n_tiles = (P.n_cols + TC_M - 1) / TC_M;
-        const unsigned grid = (unsigned)(Q.n_tiles < p->n_sm ? Q.n_tiles : p->n_sm);     // persistent: one CTA per SM
-        if (p->rows_out) k_policy_mlp_tc3<true><<<grid, T3_THREADS, tc_smem_bytes(p->act_dim), (cudaStream_t)stream>>>(Q);
-        else k_policy_mlp_tc3<false><<<grid, T3_THREADS, tc_smem_bytes(p->act_dim), (cudaStream_t)stream>>>(Q);
-        PCU_TRY(cudaGetLastError());
-        p->launches++;
-        return SWARM_OK;
+        grid = (unsigned)(Q.n_tiles < p->n_sm ? Q.n_tiles : p->n_sm);     // persistent: one CTA per SM
+        args[0] = &Q;
     }
-    if (p->precision == SWARM_POLICY_F16_TC) {
-        PolicyTcParams Q;
-        Q.base = P; Q.w16 = p->d_w16; Q.small = p->d_w + (size_t)3 * POL_HP * POL_HP; Q.debug = p->debug;
-        Q.n_tiles = (P.n_cols + TC_M - 1) / TC_M;
-        const unsigned grid = (unsigned)(Q.n_tiles < p->n_sm ? Q.n_tiles : p->n_sm);     // persistent: one CTA per SM
-        if (p->rows_out) k_policy_mlp_tc<true><<<grid, TC_THREADS, tc_smem_bytes(p->act_dim), (cudaStream_t)stream>>>(Q);
-        else k_policy_mlp_tc<false><<<grid, TC_THREADS, tc_smem_bytes(p->act_dim), (cudaStream_t)stream>>>(Q);
-        PCU_TRY(cudaGetLastError());
-        p->launches++;
-        return SWARM_OK;
-    }
-    const long ctas = (P.n_cols + POL_M - 1) / POL_M;
-    k_policy_mlp<<<(unsigned)ctas, POL_THREADS, POL_SMEM, (cudaStream_t)stream>>>(P);
-    PCU_TRY(cudaGetLastError());
+    cudaLaunchKernel(k.fn, dim3(grid), dim3(k.threads), args, k.smem, (cudaStream_t)stream);
+    PCU_TRY(cudaGetLastError());                     // returns and clears a launch error, like after a <<<>>> launch
     p->launches++;
     return SWARM_OK;
 }

@@ -48,6 +48,18 @@ __device__ __forceinline__ uint64_t pol_mix64(uint64_t seed, uint64_t a, uint64_
     z ^= z >> 31;
     return z;
 }
+// component j of column col's exploration draws (agents.py:85-93), shared by every policy kernel: a unit-variance
+// Gaussian (Box-Muller; the noise is this times P.scale) and the epsilon branch's uniform action in [-1, 1)
+__device__ __forceinline__ float pol_gauss(const PolicyParams &P, long col, int j) {
+    const uint64_t r = pol_mix64(P.seed, P.step, (uint64_t)col, (uint64_t)j);
+    const float u1 = ((float)(r >> 40) + 1.0f) * (1.0f / 16777216.0f);          // (0, 1]
+    const float u2 = (float)((r >> 16) & 0xffffffu) * (1.0f / 16777216.0f);     // [0, 1)
+    return sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2);
+}
+__device__ __forceinline__ float pol_uniform(const PolicyParams &P, long col, int j) {
+    const uint64_t r = pol_mix64(P.seed, P.step, (uint64_t)col, (uint64_t)j);
+    return (float)(r >> 40) * (2.0f / 16777216.0f) - 1.0f;
+}
 
 __device__ __forceinline__ void cp_async16(void *smem, const void *gmem) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem)), "l"(gmem) : "memory");
@@ -146,17 +158,8 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy_mlp(const PolicyParam
 #pragma unroll 4
         for (int k = 0; k < POL_HP; ++k) s = fmaf(__ldg(w4 + k), hin[k * POL_M + c], s);
         float a = tanhf(s + __ldg(P.b4 + j));                  // networks.py:29,43 (constrain_out)
-        float nz = 0.f;
-        if (P.explore == 1) {                                  // agents.py:90-93: a += scale * N(0,1), clamp
-            const uint64_t r = pol_mix64(P.seed, P.step, (uint64_t)col, (uint64_t)j);
-            const float u1 = ((float)(r >> 40) + 1.0f) * (1.0f / 16777216.0f);          // (0, 1]
-            const float u2 = (float)((r >> 16) & 0xffffffu) * (1.0f / 16777216.0f);     // [0, 1)
-            nz = sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2) * P.scale;                 // Box-Muller
-            a = fminf(fmaxf(a + nz, -1.f), 1.f);
-        } else if (P.explore == 2) {                           // agents.py:86-88: uniform action for the whole batch
-            const uint64_t r = pol_mix64(P.seed, P.step, (uint64_t)col, (uint64_t)j);
-            a = (float)(r >> 40) * (2.0f / 16777216.0f) - 1.0f;
-        }
+        if (P.explore == 1) a = fminf(fmaxf(a + pol_gauss(P, col, j) * P.scale, -1.f), 1.f);   // agents.py:90-93, clamp
+        else if (P.explore == 2) a = pol_uniform(P, col, j);  // agents.py:86-88: uniform action for the whole batch
         const long e = col / n_a; const int ag = (int)(col - e * n_a);
         P.act[(e * P.A + j) * n_a + ag] = a;
         if (P.log_pi) {
@@ -166,10 +169,7 @@ __global__ void __launch_bounds__(POL_THREADS, 1) k_policy_mlp(const PolicyParam
             else if (P.explore == 1 && j == 0) {
                 float q = 0.f;
                 for (int jj = 0; jj < P.A; ++jj) {
-                    const uint64_t r = pol_mix64(P.seed, P.step, (uint64_t)col, (uint64_t)jj);
-                    const float u1 = ((float)(r >> 40) + 1.0f) * (1.0f / 16777216.0f);
-                    const float u2 = (float)((r >> 16) & 0xffffffu) * (1.0f / 16777216.0f);
-                    const float g = sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2);            // noise / scale
+                    const float g = pol_gauss(P, col, jj);
                     q += g * g;
                 }
                 lp = -0.5f * q - (float)P.A * logf(P.scale * 2.50662827463f);
@@ -264,6 +264,179 @@ __device__ __forceinline__ void tc_commit(uint64_t *bar) {      // arrives on ba
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(s_u32(bar)) : "memory");
 }
 
+__device__ __forceinline__ void tc_expect_tx(uint64_t *bar, uint32_t bytes) {  // bar also waits for `bytes` of bulk copies
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(s_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void tc_bulk_load(void *smem, const void *gmem, uint32_t bytes, uint64_t *bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"(s_u32(smem)), "l"(gmem), "r"(bytes), "r"(s_u32(bar)) : "memory");
+}
+
+// ---- pieces shared by the two tcgen05 kernels
+// biases and output layer -> shared memory: the kernels carve sB [3][192], sW4 [A][192] and sb4 [A] back to back, the same
+// order as Q.small, so this is one copy of 3 * 192 + A * 192 + A floats
+__device__ __forceinline__ void tc_load_small(const float *small, float *sB, int A, int tid, int nthreads) {
+    for (int k = tid; k < 3 * POL_HP + A * POL_HP + A; k += nthreads) sB[k] = small[k];
+}
+
+// one warp allocates the tensor memory of this SM; the barrier also publishes everything the CTA set up before the call
+__device__ __forceinline__ uint32_t tc_tmem_alloc(uint32_t *tmem_slot, int warp) {
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"((uint32_t)TC_COLS) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    return *tmem_slot;
+}
+__device__ __forceinline__ void tc_tmem_free(uint32_t tmem, int warp) {
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"((uint32_t)TC_COLS) : "memory");
+}
+
+// pull the observations of tile nt (a contiguous run of whole envs) into the L2 while the current tile is converted
+__device__ __forceinline__ void tc_prefetch_tile(const PolicyParams &P, long nt, long n_tiles) {
+    if (nt >= n_tiles) return;
+    const int n_a = P.n_a;
+    const long e0 = nt * TC_M / n_a;
+    long e1 = (nt * TC_M + TC_M - 1) / n_a; if (e1 * n_a >= P.n_cols) e1 = (P.n_cols - 1) / n_a;
+    const size_t env_bytes = (size_t)P.K0 * n_a * sizeof(float);
+    if ((env_bytes & 15) == 0)
+        for (long ee = e0; ee <= e1; ++ee)
+            for (size_t off = 0; off < env_bytes; off += 32768) {
+                const uint32_t sz = (uint32_t)(env_bytes - off < 32768 ? env_bytes - off : 32768);
+                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(reinterpret_cast<const char *>(P.obs) + ee * env_bytes + off), "r"(sz) : "memory");
+            }
+}
+
+// loader: features k0..k0+31 of column col = agent ag of env e (zero beyond K0 and for dead columns) -> f.  ROWS: also
+// store them as the chunk of the column's replay row (swarm_policy_rows_out).
+template <bool ROWS>
+__device__ __forceinline__ void tc_load_obs32(const PolicyParams &P, long col, bool valid, long e, int ag, int k0, float (&f)[32]) {
+    if (P.obs_am && (P.K0 & 3) == 0 && k0 + 32 <= P.K0) {
+        // agent-major observations: this thread's 32 features are 128 contiguous bytes of the agent's row
+        const float4 *r4 = reinterpret_cast<const float4 *>(P.obs + col * (long)P.K0 + k0);
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+            const float4 v = valid ? __ldg(r4 + q) : make_float4(0.f, 0.f, 0.f, 0.f);
+            f[4 * q] = v.x; f[4 * q + 1] = v.y; f[4 * q + 2] = v.z; f[4 * q + 3] = v.w;
+        }
+    } else if (P.obs_am) {
+#pragma unroll
+        for (int q = 0; q < 32; ++q) {
+            const int k = k0 + q;
+            f[q] = (valid && k < P.K0) ? __ldg(P.obs + col * (long)P.K0 + k) : 0.f;
+        }
+    } else {
+#pragma unroll
+        for (int q = 0; q < 32; ++q) {
+            const int k = k0 + q;
+            f[q] = (valid && k < P.K0) ? __ldg(P.obs + (e * P.K0 + k) * P.n_a + ag) : 0.f;
+        }
+    }
+    if (ROWS && valid) {                                    // the row chunk this thread holds: 128 contiguous bytes
+        float *rw = P.rows_out + col * P.K0 + k0;
+        if ((P.K0 & 3) == 0 && k0 + 32 <= P.K0) {
+#pragma unroll
+            for (int q = 0; q < 8; ++q) reinterpret_cast<float4 *>(rw)[q] = make_float4(f[4 * q], f[4 * q + 1], f[4 * q + 2], f[4 * q + 3]);
+        } else {
+#pragma unroll
+            for (int q = 0; q < 32; ++q) if (k0 + q < P.K0) rw[q] = f[q];
+        }
+    }
+}
+
+// MMA thread: D (+)= A W^T over K = 192, twelve tcgen05.mma of K = 16 (two 16-byte k-chunks each); accumulate = false
+// makes the first one overwrite D
+__device__ __forceinline__ void tc_mma_k192(uint32_t d_tmem, uint32_t a_tmem, uint32_t wbase, bool accumulate) {
+#pragma unroll 1
+    for (int j = 0; j < POL_HP / 16; ++j) {
+        const uint64_t bdesc = tc_smem_desc(wbase + (uint32_t)j * 2u * TC_LBO);
+        const uint32_t acc = (accumulate || j > 0) ? 1u : 0u;
+        asm volatile(
+            "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+            "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, {%5, %5, %5, %5}, p;\n\t}"
+            ::"r"(d_tmem), "r"(a_tmem + j * 8), "l"(bdesc), "r"(TC_IDESC), "r"(acc), "r"(0u) : "memory");
+    }
+}
+
+// epilogue: 32 accumulator columns of this thread's row -> h = leaky_relu(acc + bias); dbg (or NULL) receives the raw
+// accumulators
+__device__ __forceinline__ void tc_bias_act32(uint32_t taddr, const float *bias, float slope, float *dbg, float (&h)[32]) {
+    uint32_t v[32];
+    TC_LD32(taddr, v);
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+    if (dbg) {
+#pragma unroll
+        for (int q = 0; q < 32; ++q) dbg[q] = __uint_as_float(v[q]);
+    }
+#pragma unroll
+    for (int q4 = 0; q4 < 8; ++q4) {
+        const float4 b4v = *reinterpret_cast<const float4 *>(bias + q4 * 4);
+        const float bb[4] = {b4v.x, b4v.y, b4v.z, b4v.w};
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const float s_ = __uint_as_float(v[q4 * 4 + u]) + bb[u];
+            h[q4 * 4 + u] = s_ > 0.f ? s_ : s_ * slope;
+        }
+    }
+}
+
+// last layer's epilogue: out[j] += the 32 h3 values times the matching output-layer weights w4 = sW4 + 32 c
+__device__ __forceinline__ void tc_out_acc32(const float (&h)[32], const float *w4, int A, float (&out)[TC_AMAX]) {
+#pragma unroll
+    for (int j = 0; j < TC_AMAX; ++j) {
+        if (j < A) {
+            float s_ = out[j];
+#pragma unroll
+            for (int q4 = 0; q4 < 8; ++q4) {
+                const float4 w = *reinterpret_cast<const float4 *>(w4 + j * POL_HP + q4 * 4);
+                s_ = fmaf(h[q4 * 4], w.x, s_); s_ = fmaf(h[q4 * 4 + 1], w.y, s_);
+                s_ = fmaf(h[q4 * 4 + 2], w.z, s_); s_ = fmaf(h[q4 * 4 + 3], w.w, s_);
+            }
+            out[j] = s_;
+        }
+    }
+}
+
+// end of a tile: the second column half hands its partial outputs to the first, which finishes the row with tanh,
+// exploration and the act / log_pi stores (same definitions as k_policy_mlp).  The barrier also orders every compute
+// thread's accumulator reads before thread 0 starts the next tile's first MMA.
+__device__ __forceinline__ void tc_finish_row(const PolicyParams &P, const float (&out)[TC_AMAX], float *s_part, const float *sb4,
+                                              int row, int half, long col, bool valid) {
+    const int A = P.A, n_a = P.n_a;
+    if (half == 1) {
+#pragma unroll
+        for (int j = 0; j < TC_AMAX; ++j) if (j < A) s_part[row * A + j] = out[j];
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    asm volatile("bar.sync 1, %0;" ::"n"(TC_CTHREADS) : "memory");
+    if (!valid || half != 0) return;
+    const long e = col / n_a; const int ag = (int)(col - e * n_a);
+    float q2 = 0.f;
+#pragma unroll
+    for (int j = 0; j < TC_AMAX; ++j) {
+        if (j >= A) break;
+        float a = tanhf((out[j] + s_part[row * A + j]) + sb4[j]);
+        if (P.explore == 1) {
+            const float g = pol_gauss(P, col, j);
+            q2 += g * g;
+            a = fminf(fmaxf(a + g * P.scale, -1.f), 1.f);
+        } else if (P.explore == 2) {
+            a = pol_uniform(P, col, j);
+        }
+        P.act[(e * A + j) * n_a + ag] = a;
+    }
+    if (P.log_pi) {
+        float lp = 0.f;
+        if (P.explore == 2) lp = -(float)A * 0.69314718056f;
+        else if (P.explore == 1) lp = -0.5f * q2 - (float)A * logf(P.scale * 2.50662827463f);
+        P.log_pi[e * n_a + ag] = lp;
+    }
+}
+
 template <bool ROWS>   // ROWS: the loaders also write every agent's observation as a replay row (swarm_policy_rows_out)
 __global__ void __launch_bounds__(TC_THREADS, 1) k_policy_mlp_tc(const PolicyTcParams Q) {
     extern __shared__ __align__(128) unsigned char tsm[];
@@ -279,32 +452,18 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_policy_mlp_tc(const PolicyTcP
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bar_free + 2);
     const PolicyParams &P = Q.base;
     const int tid = threadIdx.x, warp = tid >> 5;
-    const int A = P.A, n_a = P.n_a;
+    const int n_a = P.n_a;
 
     if (tid == 0) {
         tc_mbar_init(bar_w, 1); tc_mbar_init(bar_mma, 1);
         tc_mbar_init(&bar_full[0], TC_LOADERS * TC_M); tc_mbar_init(&bar_full[1], TC_LOADERS * TC_M);
         tc_mbar_init(&bar_free[0], 1); tc_mbar_init(&bar_free[1], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(s_u32(bar_w)), "r"(3u * TC_W_BYTES) : "memory");
-        for (int l = 0; l < 3; ++l)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(s_u32(sW + l * TC_W_BYTES)), "l"(Q.w16 + (size_t)l * TC_W_BYTES), "r"((uint32_t)TC_W_BYTES), "r"(s_u32(bar_w)) : "memory");
+        tc_expect_tx(bar_w, 3u * TC_W_BYTES);
+        for (int l = 0; l < 3; ++l) tc_bulk_load(sW + l * TC_W_BYTES, Q.w16 + (size_t)l * TC_W_BYTES, (uint32_t)TC_W_BYTES, bar_w);
     }
-    for (int k = tid; k < 3 * POL_HP + A * POL_HP + A; k += TC_THREADS) { // biases + output layer: sB, sW4 (A rows), sb4
-        const float v = Q.small[k];
-        if (k < 3 * POL_HP) sB[k] = v;
-        else if (k < 3 * POL_HP + A * POL_HP) sW4[k - 3 * POL_HP] = v;
-        else sb4[k - 3 * POL_HP - A * POL_HP] = v;
-    }
-    if (warp == 0) {                                                     // one warp allocates the tensor memory of this SM
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"((uint32_t)TC_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem = *tmem_slot;
+    tc_load_small(Q.small, sB, P.A, tid, TC_THREADS);
+    const uint32_t tmem = tc_tmem_alloc(tmem_slot, warp);
     const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);   // a warp reaches the TMEM lane quadrant warp % 4
     const int row = tid & (TC_M - 1);                                    // TMEM lane = agent of the tile
 
@@ -314,63 +473,19 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_policy_mlp_tc(const PolicyTcP
 #pragma unroll 1
         for (long tile = blockIdx.x; tile < Q.n_tiles; tile += gridDim.x, ++it) {
             const int b = it & 1;
-            if (tid == TC_CTHREADS) {  // pull the NEXT tile's observations (a contiguous run of whole envs) into the L2 while this one is converted
-                const long nt = tile + gridDim.x;
-                if (nt < Q.n_tiles) {
-                    const long e0 = nt * TC_M / n_a;
-                    long e1 = (nt * TC_M + TC_M - 1) / n_a; if (e1 * n_a >= P.n_cols) e1 = (P.n_cols - 1) / n_a;
-                    const size_t env_bytes = (size_t)P.K0 * n_a * sizeof(float);
-                    if ((env_bytes & 15) == 0)
-                        for (long ee = e0; ee <= e1; ++ee)
-                            for (size_t off = 0; off < env_bytes; off += 32768) {
-                                const uint32_t sz = (uint32_t)(env_bytes - off < 32768 ? env_bytes - off : 32768);
-                                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(reinterpret_cast<const char *>(P.obs) + ee * env_bytes + off), "r"(sz) : "memory");
-                            }
-                }
-            }
+            if (tid == TC_CTHREADS) tc_prefetch_tile(P, tile + gridDim.x, Q.n_tiles);
             if (it >= 2) tc_mbar_wait(&bar_free[b], (uint32_t)((it >> 1) - 1) & 1u);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             const long col = tile * TC_M + row;
             const bool valid = col < P.n_cols;
             const long e = valid ? col / n_a : 0; const int ag = valid ? (int)(col - e * n_a) : 0;
-            const float *orow = P.obs + e * (long)P.K0 * n_a + ag;
             const uint32_t abase = lane_base + (b ? TC_COL_A1 : TC_COL_A);
             constexpr int FPL = POL_HP / TC_LOADERS;                     // features per loader thread
             const int k_lo = ((warp - 4 * TC_EPI) >> 2) * FPL;
 #pragma unroll 1
             for (int c = 0; c < FPL / 32; ++c) {                         // 32 loads in flight per thread and batch (register budget: 512 threads)
                 float f[32];
-                if (P.obs_am && (P.K0 & 3) == 0 && k_lo + c * 32 + 32 <= P.K0) {
-                    // agent-major observations: this thread's 32 features are 128 contiguous bytes of the agent's row
-                    const float4 *r4 = reinterpret_cast<const float4 *>(P.obs + col * (long)P.K0 + k_lo + c * 32);
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) {
-                        const float4 v = valid ? __ldg(r4 + q) : make_float4(0.f, 0.f, 0.f, 0.f);
-                        f[4 * q] = v.x; f[4 * q + 1] = v.y; f[4 * q + 2] = v.z; f[4 * q + 3] = v.w;
-                    }
-                } else if (P.obs_am) {
-#pragma unroll
-                    for (int q = 0; q < 32; ++q) {
-                        const int k = k_lo + c * 32 + q;
-                        f[q] = (valid && k < P.K0) ? __ldg(P.obs + col * (long)P.K0 + k) : 0.f;
-                    }
-                } else {
-#pragma unroll
-                    for (int q = 0; q < 32; ++q) {
-                        const int k = k_lo + c * 32 + q;
-                        f[q] = (valid && k < P.K0) ? __ldg(orow + (long)k * n_a) : 0.f;
-                    }
-                }
-                if (ROWS && valid) {                                // the row chunk this thread holds: 128 contiguous bytes
-                    float *rw = P.rows_out + col * P.K0 + k_lo + c * 32;
-                    if ((P.K0 & 3) == 0 && k_lo + c * 32 + 32 <= P.K0) {
-#pragma unroll
-                        for (int q = 0; q < 8; ++q) reinterpret_cast<float4 *>(rw)[q] = make_float4(f[4 * q], f[4 * q + 1], f[4 * q + 2], f[4 * q + 3]);
-                    } else {
-#pragma unroll
-                        for (int q = 0; q < 32; ++q) if (k_lo + c * 32 + q < P.K0) rw[q] = f[q];
-                    }
-                }
+                tc_load_obs32<ROWS>(P, col, valid, e, ag, k_lo + c * 32, f);
                 uint32_t r[16];
 #pragma unroll
                 for (int q = 0; q < 16; ++q) r[q] = pack_h2(f[2 * q], f[2 * q + 1]);
@@ -391,7 +506,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_policy_mlp_tc(const PolicyTcP
             const uint32_t acol = b ? TC_COL_A1 : TC_COL_A;
             const long col = tile * TC_M + row;
             const bool valid = col < P.n_cols;
-            const long e = valid ? col / n_a : 0; const int ag = valid ? (int)(col - e * n_a) : 0;
+            float *dbg = Q.debug && valid ? Q.debug + col * POL_HP : nullptr;
             float out[TC_AMAX];
 #pragma unroll
             for (int j = 0; j < TC_AMAX; ++j) out[j] = 0.f;
@@ -405,104 +520,31 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_policy_mlp_tc(const PolicyTcP
                     if (it == 0 && layer == 0) tc_mbar_wait(bar_w, 0);
                     if (layer == 0) tc_mbar_wait(&bar_full[b], (uint32_t)(it >> 1) & 1u);
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                    const uint32_t wbase = s_u32(sW + layer * TC_W_BYTES);
-#pragma unroll 1
-                    for (int j = 0; j < POL_HP / 16; ++j) {              // K = 16 per instruction: two 16-byte k-chunks
-                        const uint64_t bdesc = tc_smem_desc(wbase + (uint32_t)j * 2u * TC_LBO);
-                        const uint32_t acc = j > 0 ? 1u : 0u;
-                        asm volatile(
-                            "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                            "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, {%5, %5, %5, %5}, p;\n\t}"
-                            ::"r"(tmem + TC_COL_D), "r"(tmem + acol + j * 8), "l"(bdesc), "r"(TC_IDESC), "r"(acc), "r"(0u) : "memory");
-                    }
+                    tc_mma_k192(tmem + TC_COL_D, tmem + acol, s_u32(sW + layer * TC_W_BYTES), false);
                     tc_commit(bar_mma);
                     if (layer == 2) tc_commit(&bar_free[b]);             // buffer b may be refilled once these MMAs have retired
                 }
                 tc_mbar_wait(bar_mma, par_mma); par_mma ^= 1u;
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                const float *bias = sB + layer * POL_HP;
 #pragma unroll 1
                 for (int c = half * (POL_HP / 32 / TC_EPI); c < (half + 1) * (POL_HP / 32 / TC_EPI); ++c) {   // 32 accumulator columns at a time
-                    uint32_t v[32];
-                    TC_LD32(lane_base + TC_COL_D + c * 32, v);
-                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                    if (Q.debug && layer == 0 && valid) {
-#pragma unroll
-                        for (int q = 0; q < 32; ++q) Q.debug[col * POL_HP + c * 32 + q] = __uint_as_float(v[q]);
-                    }
                     float h[32];
-#pragma unroll
-                    for (int q4 = 0; q4 < 8; ++q4) {
-                        const float4 b4v = *reinterpret_cast<const float4 *>(bias + c * 32 + q4 * 4);
-                        const float bb[4] = {b4v.x, b4v.y, b4v.z, b4v.w};
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) {
-                            const float s_ = __uint_as_float(v[q4 * 4 + u]) + bb[u];
-                            h[q4 * 4 + u] = s_ > 0.f ? s_ : s_ * P.slope;
-                        }
-                    }
+                    tc_bias_act32(lane_base + TC_COL_D + c * 32, sB + layer * POL_HP + c * 32, P.slope, layer == 0 && dbg ? dbg + c * 32 : nullptr, h);
                     if (layer < 2) {
                         uint32_t r[16];
 #pragma unroll
                         for (int q = 0; q < 16; ++q) r[q] = pack_h2(h[2 * q], h[2 * q + 1]);
                         TC_ST16(lane_base + acol + c * 16, r);
                     } else {
-#pragma unroll
-                        for (int j = 0; j < TC_AMAX; ++j) {
-                            if (j < A) {
-                                float s_ = out[j];
-#pragma unroll
-                                for (int q4 = 0; q4 < 8; ++q4) {
-                                    const float4 w = *reinterpret_cast<const float4 *>(sW4 + j * POL_HP + c * 32 + q4 * 4);
-                                    s_ = fmaf(h[q4 * 4], w.x, s_); s_ = fmaf(h[q4 * 4 + 1], w.y, s_);
-                                    s_ = fmaf(h[q4 * 4 + 2], w.z, s_); s_ = fmaf(h[q4 * 4 + 3], w.w, s_);
-                                }
-                                out[j] = s_;
-                            }
-                        }
+                        tc_out_acc32(h, sW4 + c * 32, P.A, out);
                     }
                 }
                 if (layer < 2) asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
             }
-            if (half == 1) {                                             // the first half finishes the row
-#pragma unroll
-                for (int j = 0; j < TC_AMAX; ++j) if (j < A) s_part[row * A + j] = out[j];
-            }
-            // every compute thread has read its accumulator row before thread 0 may start the next tile's first MMA
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            asm volatile("bar.sync 1, %0;" ::"n"(TC_CTHREADS) : "memory");
-            // ---- tanh, exploration, outputs (same definitions as k_policy_mlp)
-            if (valid && half == 0) {
-                float q2 = 0.f;
-#pragma unroll
-                for (int j = 0; j < TC_AMAX; ++j) {
-                    if (j >= A) break;
-                    float a = tanhf((out[j] + s_part[row * A + j]) + sb4[j]);
-                    if (P.explore == 1) {
-                        const uint64_t r = pol_mix64(P.seed, P.step, (uint64_t)col, (uint64_t)j);
-                        const float u1 = ((float)(r >> 40) + 1.0f) * (1.0f / 16777216.0f);
-                        const float u2 = (float)((r >> 16) & 0xffffffu) * (1.0f / 16777216.0f);
-                        const float g = sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2);
-                        q2 += g * g;
-                        a = fminf(fmaxf(a + g * P.scale, -1.f), 1.f);
-                    } else if (P.explore == 2) {
-                        const uint64_t r = pol_mix64(P.seed, P.step, (uint64_t)col, (uint64_t)j);
-                        a = (float)(r >> 40) * (2.0f / 16777216.0f) - 1.0f;
-                    }
-                    P.act[(e * A + j) * n_a + ag] = a;
-                }
-                if (P.log_pi) {
-                    float lp = 0.f;
-                    if (P.explore == 2) lp = -(float)A * 0.69314718056f;
-                    else if (P.explore == 1) lp = -0.5f * q2 - (float)A * logf(P.scale * 2.50662827463f);
-                    P.log_pi[e * n_a + ag] = lp;
-                }
-            }
+            tc_finish_row(P, out, s_part, sb4, row, half, col, valid);
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"((uint32_t)TC_COLS) : "memory");
+    tc_tmem_free(tmem, warp);
 }
 
 // =====================================================================================================
@@ -544,7 +586,7 @@ __global__ void __launch_bounds__(T3_THREADS, 1) k_policy_mlp_tc3(const PolicyTc
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bar_free + 3);
     const PolicyParams &P = Q.base;
     const int tid = threadIdx.x, warp = tid >> 5;
-    const int A = P.A, n_a = P.n_a;
+    const int n_a = P.n_a;
     const long my_tiles = (Q.n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x;
 
     if (tid == 0) {
@@ -552,20 +594,8 @@ __global__ void __launch_bounds__(T3_THREADS, 1) k_policy_mlp_tc3(const PolicyTc
         for (int k = 0; k < 3; ++k) { tc_mbar_init(&bar_full[k], 1); tc_mbar_init(&bar_free[k], 1); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    for (int k = tid; k < 3 * POL_HP + A * POL_HP + A; k += T3_THREADS) {
-        const float v = Q.small[k];
-        if (k < 3 * POL_HP) sB[k] = v;
-        else if (k < 3 * POL_HP + A * POL_HP) sW4[k - 3 * POL_HP] = v;
-        else sb4[k - 3 * POL_HP - A * POL_HP] = v;
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"((uint32_t)TC_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem = *tmem_slot;
+    tc_load_small(Q.small, sB, P.A, tid, T3_THREADS);
+    const uint32_t tmem = tc_tmem_alloc(tmem_slot, warp);
     const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
     const int row = tid & (TC_M - 1);
 
@@ -577,10 +607,8 @@ __global__ void __launch_bounds__(T3_THREADS, 1) k_policy_mlp_tc3(const PolicyTc
             for (long k = 0; k < n_chunks; ++k) {
                 const int slot = (int)(k % 3);
                 if (k >= 3) tc_mbar_wait(&bar_free[slot], (uint32_t)((k / 3 - 1) & 1));
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(s_u32(&bar_full[slot])), "r"((uint32_t)TC_W_BYTES) : "memory");
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                             ::"r"(s_u32(sW + slot * TC_W_BYTES)), "l"(Q.w16 + (size_t)(k % 6) * TC_W_BYTES), "r"((uint32_t)TC_W_BYTES),
-                               "r"(s_u32(&bar_full[slot])) : "memory");
+                tc_expect_tx(&bar_full[slot], (uint32_t)TC_W_BYTES);
+                tc_bulk_load(sW + slot * TC_W_BYTES, Q.w16 + (size_t)(k % 6) * TC_W_BYTES, (uint32_t)TC_W_BYTES, &bar_full[slot]);
             }
         }
     } else if (warp >= 4 * TC_EPI) {
@@ -588,62 +616,18 @@ __global__ void __launch_bounds__(T3_THREADS, 1) k_policy_mlp_tc3(const PolicyTc
         int it = 0;
 #pragma unroll 1
         for (long tile = blockIdx.x; tile < Q.n_tiles; tile += gridDim.x, ++it) {
-            if (tid == TC_CTHREADS) {                                    // pull the NEXT tile's observations into the L2
-                const long nt = tile + gridDim.x;
-                if (nt < Q.n_tiles) {
-                    const long e0 = nt * TC_M / n_a;
-                    long e1 = (nt * TC_M + TC_M - 1) / n_a; if (e1 * n_a >= P.n_cols) e1 = (P.n_cols - 1) / n_a;
-                    const size_t env_bytes = (size_t)P.K0 * n_a * sizeof(float);
-                    if ((env_bytes & 15) == 0)
-                        for (long ee = e0; ee <= e1; ++ee)
-                            for (size_t off = 0; off < env_bytes; off += 32768) {
-                                const uint32_t sz = (uint32_t)(env_bytes - off < 32768 ? env_bytes - off : 32768);
-                                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(reinterpret_cast<const char *>(P.obs) + ee * env_bytes + off), "r"(sz) : "memory");
-                            }
-                }
-            }
+            if (tid == TC_CTHREADS) tc_prefetch_tile(P, tile + gridDim.x, Q.n_tiles);
             if (it >= 1) tc_mbar_wait(bar_afree, (uint32_t)(it - 1) & 1u);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             const long col = tile * TC_M + row;
             const bool valid = col < P.n_cols;
             const long e = valid ? col / n_a : 0; const int ag = valid ? (int)(col - e * n_a) : 0;
-            const float *orow = P.obs + e * (long)P.K0 * n_a + ag;
             constexpr int FPL = POL_HP / TC_LOADERS;
             const int k_lo = ((warp - 4 * TC_EPI) >> 2) * FPL;
 #pragma unroll 1
             for (int c = 0; c < FPL / 32; ++c) {
                 float f[32];
-                if (P.obs_am && (P.K0 & 3) == 0 && k_lo + c * 32 + 32 <= P.K0) {
-                    // agent-major observations: this thread's 32 features are 128 contiguous bytes of the agent's row
-                    const float4 *r4 = reinterpret_cast<const float4 *>(P.obs + col * (long)P.K0 + k_lo + c * 32);
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) {
-                        const float4 v = valid ? __ldg(r4 + q) : make_float4(0.f, 0.f, 0.f, 0.f);
-                        f[4 * q] = v.x; f[4 * q + 1] = v.y; f[4 * q + 2] = v.z; f[4 * q + 3] = v.w;
-                    }
-                } else if (P.obs_am) {
-#pragma unroll
-                    for (int q = 0; q < 32; ++q) {
-                        const int k = k_lo + c * 32 + q;
-                        f[q] = (valid && k < P.K0) ? __ldg(P.obs + col * (long)P.K0 + k) : 0.f;
-                    }
-                } else {
-#pragma unroll
-                    for (int q = 0; q < 32; ++q) {
-                        const int k = k_lo + c * 32 + q;
-                        f[q] = (valid && k < P.K0) ? __ldg(orow + (long)k * n_a) : 0.f;
-                    }
-                }
-                if (ROWS && valid) {
-                    float *rw = P.rows_out + col * P.K0 + k_lo + c * 32;
-                    if ((P.K0 & 3) == 0 && k_lo + c * 32 + 32 <= P.K0) {
-#pragma unroll
-                        for (int q = 0; q < 8; ++q) reinterpret_cast<float4 *>(rw)[q] = make_float4(f[4 * q], f[4 * q + 1], f[4 * q + 2], f[4 * q + 3]);
-                    } else {
-#pragma unroll
-                        for (int q = 0; q < 32; ++q) if (k_lo + c * 32 + q < P.K0) rw[q] = f[q];
-                    }
-                }
+                tc_load_obs32<ROWS>(P, col, valid, e, ag, k_lo + c * 32, f);
                 uint32_t rh[16], rl[16];
 #pragma unroll
                 for (int q = 0; q < 16; ++q) split_h2(f[2 * q], f[2 * q + 1], rh[q], rl[q]);
@@ -664,7 +648,7 @@ __global__ void __launch_bounds__(T3_THREADS, 1) k_policy_mlp_tc3(const PolicyTc
         for (long tile = blockIdx.x; tile < Q.n_tiles; tile += gridDim.x, ++it) {
             const long col = tile * TC_M + row;
             const bool valid = col < P.n_cols;
-            const long e = valid ? col / n_a : 0; const int ag = valid ? (int)(col - e * n_a) : 0;
+            float *dbg = Q.debug && valid ? Q.debug + col * POL_HP : nullptr;
             float out[TC_AMAX];
 #pragma unroll
             for (int j = 0; j < TC_AMAX; ++j) out[j] = 0.f;
@@ -682,17 +666,7 @@ __global__ void __launch_bounds__(T3_THREADS, 1) k_policy_mlp_tc3(const PolicyTc
                         const long kk = kc + (g == 2 ? 1 : 0);
                         const int slot = (int)(kk % 3);
                         if (g != 1) { tc_mbar_wait(&bar_full[slot], (uint32_t)((kk / 3) & 1)); asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-                        const uint32_t wbase = s_u32(sW + slot * TC_W_BYTES);
-                        const uint32_t acol = (g == 1) ? T3_COL_AL : T3_COL_AH;
-#pragma unroll 1
-                        for (int j = 0; j < POL_HP / 16; ++j) {
-                            const uint64_t bdesc = tc_smem_desc(wbase + (uint32_t)j * 2u * TC_LBO);
-                            const uint32_t acc = (g > 0 || j > 0) ? 1u : 0u;
-                            asm volatile(
-                                "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                                "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, {%5, %5, %5, %5}, p;\n\t}"
-                                ::"r"(tmem + TC_COL_D), "r"(tmem + acol + j * 8), "l"(bdesc), "r"(TC_IDESC), "r"(acc), "r"(0u) : "memory");
-                        }
+                        tc_mma_k192(tmem + TC_COL_D, tmem + (g == 1 ? T3_COL_AL : T3_COL_AH), s_u32(sW + slot * TC_W_BYTES), g > 0);
                         if (g >= 1) tc_commit(&bar_free[slot]);          // H after its second use, L after its only use
                     }
                     kc += 2;
@@ -701,27 +675,10 @@ __global__ void __launch_bounds__(T3_THREADS, 1) k_policy_mlp_tc3(const PolicyTc
                 }
                 tc_mbar_wait(bar_mma, par_mma); par_mma ^= 1u;
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                const float *bias = sB + layer * POL_HP;
 #pragma unroll 1
                 for (int c = half * (POL_HP / 32 / TC_EPI); c < (half + 1) * (POL_HP / 32 / TC_EPI); ++c) {
-                    uint32_t v[32];
-                    TC_LD32(lane_base + TC_COL_D + c * 32, v);
-                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                    if (Q.debug && layer == 0 && valid) {
-#pragma unroll
-                        for (int q = 0; q < 32; ++q) Q.debug[col * POL_HP + c * 32 + q] = __uint_as_float(v[q]);
-                    }
                     float h[32];
-#pragma unroll
-                    for (int q4 = 0; q4 < 8; ++q4) {
-                        const float4 b4v = *reinterpret_cast<const float4 *>(bias + c * 32 + q4 * 4);
-                        const float bb[4] = {b4v.x, b4v.y, b4v.z, b4v.w};
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) {
-                            const float s_ = __uint_as_float(v[q4 * 4 + u]) + bb[u];
-                            h[q4 * 4 + u] = s_ > 0.f ? s_ : s_ * P.slope;
-                        }
-                    }
+                    tc_bias_act32(lane_base + TC_COL_D + c * 32, sB + layer * POL_HP + c * 32, P.slope, layer == 0 && dbg ? dbg + c * 32 : nullptr, h);
                     if (layer < 2) {
                         uint32_t rh[16], rl[16];
 #pragma unroll
@@ -729,60 +686,15 @@ __global__ void __launch_bounds__(T3_THREADS, 1) k_policy_mlp_tc3(const PolicyTc
                         TC_ST16(lane_base + T3_COL_AH + c * 16, rh);
                         TC_ST16(lane_base + T3_COL_AL + c * 16, rl);
                     } else {
-#pragma unroll
-                        for (int j = 0; j < TC_AMAX; ++j) {
-                            if (j < A) {
-                                float s_ = out[j];
-#pragma unroll
-                                for (int q4 = 0; q4 < 8; ++q4) {
-                                    const float4 w = *reinterpret_cast<const float4 *>(sW4 + j * POL_HP + c * 32 + q4 * 4);
-                                    s_ = fmaf(h[q4 * 4], w.x, s_); s_ = fmaf(h[q4 * 4 + 1], w.y, s_);
-                                    s_ = fmaf(h[q4 * 4 + 2], w.z, s_); s_ = fmaf(h[q4 * 4 + 3], w.w, s_);
-                                }
-                                out[j] = s_;
-                            }
-                        }
+                        tc_out_acc32(h, sW4 + c * 32, P.A, out);
                     }
                 }
                 if (layer < 2) asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
             }
-            if (half == 1) {
-#pragma unroll
-                for (int j = 0; j < TC_AMAX; ++j) if (j < A) s_part[row * A + j] = out[j];
-            }
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            asm volatile("bar.sync 1, %0;" ::"n"(TC_CTHREADS) : "memory");
-            if (valid && half == 0) {
-                float q2 = 0.f;
-#pragma unroll
-                for (int j = 0; j < TC_AMAX; ++j) {
-                    if (j >= A) break;
-                    float a = tanhf((out[j] + s_part[row * A + j]) + sb4[j]);
-                    if (P.explore == 1) {
-                        const uint64_t r = pol_mix64(P.seed, P.step, (uint64_t)col, (uint64_t)j);
-                        const float u1 = ((float)(r >> 40) + 1.0f) * (1.0f / 16777216.0f);
-                        const float u2 = (float)((r >> 16) & 0xffffffu) * (1.0f / 16777216.0f);
-                        const float g = sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2);
-                        q2 += g * g;
-                        a = fminf(fmaxf(a + g * P.scale, -1.f), 1.f);
-                    } else if (P.explore == 2) {
-                        const uint64_t r = pol_mix64(P.seed, P.step, (uint64_t)col, (uint64_t)j);
-                        a = (float)(r >> 40) * (2.0f / 16777216.0f) - 1.0f;
-                    }
-                    P.act[(e * A + j) * n_a + ag] = a;
-                }
-                if (P.log_pi) {
-                    float lp = 0.f;
-                    if (P.explore == 2) lp = -(float)A * 0.69314718056f;
-                    else if (P.explore == 1) lp = -0.5f * q2 - (float)A * logf(P.scale * 2.50662827463f);
-                    P.log_pi[e * n_a + ag] = lp;
-                }
-            }
+            tc_finish_row(P, out, s_part, sb4, row, half, col, valid);
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"((uint32_t)TC_COLS) : "memory");
+    tc_tmem_free(tmem, warp);
 }
 
 }  // namespace swarm

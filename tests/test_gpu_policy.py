@@ -54,12 +54,25 @@ def test_policy_matches_torch_fp32(E, n_a, D, H, A):
     assert pol.launch_count == 2
 
 
+PRECISIONS = ["fp32", "f16_tc", "f16x3_tc"]
+
+
 def test_exploration_noise_statistics_and_log_prob():
+    _check_exploration("fp32")
+
+
+@pytest.mark.parametrize("prec", ["f16_tc", "f16x3_tc"])
+def test_exploration_noise_statistics_and_log_prob_tensor_cores(prec):
+    """The tensor-core kernels' own exploration tail, held to the fp32 kernel's statistics and tolerances."""
+    _check_exploration(prec)
+
+
+def _check_exploration(prec):
     E, n_a, D, H, A = 2048, 30, 192, 180, 2
     torch.manual_seed(0)
     ref = RefMLP(D, A, H)
     obs = torch.randn(E, D, n_a, device="cuda") * 0.3
-    pol = DevicePolicy(D, A, H, noise_scale=0.1, epsilon=0.0, seed=7).load_state_dict(ref.state_dict())
+    pol = DevicePolicy(D, A, H, noise_scale=0.1, epsilon=0.0, seed=7, precision=prec).load_state_dict(ref.state_dict())
     clean, _ = pol.step(obs)
     noisy, log_pi = pol.step(obs, explore=True)
     noise = (noisy - clean).double()
@@ -78,6 +91,50 @@ def test_exploration_noise_statistics_and_log_prob():
     uni, lp = pol.step(obs, explore=True)
     assert float(uni.min()) >= -1 and float(uni.max()) <= 1 and abs(float(uni.mean())) < 2e-3
     assert abs(float(uni.double().var()) - 1 / 3) < 2e-3 and torch.allclose(lp, torch.full_like(lp, -A * np.log(2.0)))
+
+
+@pytest.mark.parametrize("A", [2, 3])
+def test_exploration_draws_are_identical_across_kernels(A):
+    """The epsilon branch's actions and log_pi and the Gaussian branch's log_pi do not depend on the network: the generator
+    is keyed by (seed, step, column, component) and every kernel sums the squared draws in the same order.  So all three
+    kernels must write the same bits."""
+    E, n_a, D, H = 67, 30, 192, 180
+    torch.manual_seed(5)
+    ref = RefMLP(D, A, H)
+    obs = torch.randn(E, D, n_a, device="cuda")
+    got = {}
+    for prec in PRECISIONS:
+        pol = DevicePolicy(D, A, H, noise_scale=0.2, epsilon=0.0, seed=3, precision=prec).load_state_dict(ref.state_dict())
+        _, lp_gauss = pol.step(obs, explore=True)          # step 0: Gaussian branch
+        pol.epsilon = 1.0
+        uni, lp_uni = pol.step(obs, explore=True)          # step 1: epsilon branch
+        got[prec] = (lp_gauss, uni, lp_uni)
+    for prec in PRECISIONS[1:]:
+        for want, have in zip(got["fp32"], got[prec]):
+            assert torch.equal(want, have), prec
+    assert not torch.equal(got["fp32"][1][:, 0], got["fp32"][1][:, 1])     # components draw different numbers
+
+
+@pytest.mark.parametrize("prec", PRECISIONS)
+@pytest.mark.parametrize("agent_major", [False, True])
+@pytest.mark.parametrize("E,n_a,D", [(67, 30, 192), (5, 7, 190), (2, 33, 100), (700, 30, 188)])
+def test_rows_out_is_the_transposed_observation(prec, agent_major, E, n_a, D):
+    """swarm_policy_rows_out: every agent's observation row, bit for bit, for both input layouts.  obs_dim 190 (not a multiple
+    of 4) and 100 (not a multiple of 32) take the loaders' scalar tails; 700 x 30 agents = 165 tiles > 148 SMs.  Writing the
+    rows does not change the actions."""
+    H, A = 180, 2
+    torch.manual_seed(E + D)
+    ref = RefMLP(D, A, H)
+    obs = torch.randn(E, D, n_a, device="cuda")
+    rows_want = obs.transpose(1, 2).reshape(E * n_a, D)
+    x = rows_want.reshape(E, n_a, D).contiguous() if agent_major else obs
+    pol = DevicePolicy(D, A, H, precision=prec).load_state_dict(ref.state_dict())
+    rows = torch.full((E * n_a, D), float("nan"), device="cuda")
+    act, _ = pol.step(x, rows_out=rows, agent_major=agent_major)
+    act = act.clone()
+    assert torch.equal(rows, rows_want)
+    act_plain, _ = pol.step(x, agent_major=agent_major)
+    assert torch.equal(act, act_plain)
 
 
 def _f16_pipeline(ref, x):

@@ -1,4 +1,7 @@
-"""Times k_policy_mlp at the BASELINE config-3 shape (65536 envs x 30 agents) with CUDA events (profiling aid)."""
+"""Times one policy kernel at the BASELINE config-3 shape (65536 envs x 30 agents) with CUDA events (profiling aid).
+
+usage: bench_policy.py [fp32 | f16_tc | f16x3_tc] [am]
+The precision picks k_policy_mlp, k_policy_mlp_tc or k_policy_mlp_tc3; `am` passes agent-major observation rows."""
 import json, os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
