@@ -2,7 +2,7 @@
  * swarm_b200.h — C ABI of the B200-native batched simulator for the MARL-LLM assembly env step path.
  *
  * One shared library (marl_llm_b200/lib/libswarm_b200.so, also reachable as libAssemblyEnv.so)
- * exports two groups of entry points, all `extern "C"`, plain pointers and sizes only:
+ * exports these groups of entry points (the first two below; (3)-(5) further down), all `extern "C"`, plain pointers and sizes only:
  *
  *  (1) LEGACY, stateless, HOST pointers — the five symbols the reference Python env binds with ctypes
  *      (cus_gym/gym/envs/customized_envs/envs_cplus/c_lib.py:11-22 loads build/libAssemblyEnv.so;
@@ -430,6 +430,36 @@ int swarm_policy_rows_out(swarm_policy *p, float *rows_dev);
  * simulator created with SWARM_OBS_AGENT_MAJOR (each loader thread then reads 128 contiguous bytes instead of 32 strided words),
  * e.g. a slot of a time-indexed replay ring the simulator wrote its observation into directly. */
 int swarm_policy_obs_layout(swarm_policy *p, int agent_major);
+
+/* ============================================================================================
+ * (5) State store: save env states of a batched handle on the device and load them back into the same or another handle,
+ *     one state into many envs (clone = save + load with a repeated slot).  Every step after a load is bit-identical to the
+ *     run the saved envs would have continued (DESIGN.md §11).
+ * ============================================================================================ */
+typedef struct swarm_state_store swarm_state_store;   /* opaque, library-owned device memory on the handle's device */
+
+/* `capacity` slots, each holding one env's complete state, for handles of sim's configuration: every field of swarm_config
+ * except num_envs, the device included.  Flocking handles: SWARM_ERR_UNSUPPORTED.  The store has its own lifetime. */
+int swarm_state_store_create(const swarm_sim *sim, int64_t capacity, swarm_state_store **out);
+int swarm_state_store_destroy(swarm_state_store *st);
+/* bytes of one slot (the layout is private to the library); 0 when st is NULL */
+int64_t swarm_state_slot_bytes(const swarm_state_store *st);
+/* A slot holds p, dp, the padded grid row, word_box, frame, n_g, in_thresh, the library pose and shape id, nearest_cell,
+ * neighbor_index, in_flags, obs (of the current observation buffer), reward; with want_prior the prior of the current state and
+ * the prior the last step returned; with emit_indices sensed_index and occupied_index (done is constant).  The store also keeps,
+ * per slot on the host, the source env's match record, whether the source's prior was valid and the fingerprint of the source's
+ * shape library.
+ *
+ * swarm_state_save: slot slots[k] <- env env_ids[k] of sim.  env_ids, slots: HOST [count]; slots distinct; sim observed.
+ * swarm_state_load: env env_ids[k] of sim <- slot slots[k].  env_ids distinct, slots filled and may repeat.  sim may be any handle
+ * of the store's configuration; one that was never observed only when env_ids covers every env (it is observed afterwards).
+ * A slot saved under another shape library (swarm_set_shapes) is restored as unmatched: the general scan serves that env, with the
+ * same results.  A slot whose prior was stale (state changed behind the handle's back) makes the next step recompute the prior.
+ * Every argument is checked before anything is launched (SWARM_ERR_INVALID; handle and store unchanged).  Stream-ordered, no host
+ * synchronisation and no host-to-device copy: the pairs travel in the kernel parameters (one launch per 2048 pairs, counted in
+ * sim's swarm_launch_count); the caller may free the host arrays when the call returns. */
+int swarm_state_save(swarm_sim *sim, swarm_state_store *st, const int32_t *env_ids, const int32_t *slots, int32_t count, void *stream);
+int swarm_state_load(swarm_sim *sim, swarm_state_store *st, const int32_t *slots, const int32_t *env_ids, int32_t count, void *stream);
 
 const char *swarm_last_error(void);
 int swarm_abi_version(void);

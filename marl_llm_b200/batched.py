@@ -32,6 +32,10 @@ def r_avoid_for(n_a, n_gs, l_cells):
 
 
 class BatchedAssemblySim:
+    """E assembly envs on one device.  To save env states and load them back into this or another handle of the same
+    configuration (several policies from the same start states, branching rollouts, one env cloned into others), use
+    marl_llm_b200.state_store.StateStore rather than copying the buffers by hand."""
+
     def __init__(self, num_envs, n_a, n_g_max, r_avoid, *, device=0, out_dtype=torch.float32, emit_indices=False,
                  want_prior=True, is_con_self_state=True, is_periodic=False, d_sen=0.4, size_a=0.035, k_ball=30.0,
                  k_wall=100.0, c_wall=5.0, dt=0.1, vel_max=0.8, mass=1.0, half_width=2.4, half_height=2.4,

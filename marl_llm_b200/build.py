@@ -9,7 +9,7 @@ import subprocess
 PKG = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(PKG, "csrc", "swarm_abi.cu")
 SRCS = [SRC, os.path.join(PKG, "csrc", "rollout_abi.cu"), os.path.join(PKG, "csrc", "policy_abi.cu")]
-DEPS = SRCS + [os.path.join(PKG, "csrc", "swarm_kernels.cuh"), os.path.join(PKG, "csrc", "render_kernels.cuh"), os.path.join(PKG, "csrc", "rollout_kernels.cuh"), os.path.join(PKG, "csrc", "policy_kernels.cuh"),
+DEPS = SRCS + [os.path.join(PKG, "csrc", "swarm_kernels.cuh"), os.path.join(PKG, "csrc", "render_kernels.cuh"), os.path.join(PKG, "csrc", "state_kernels.cuh"), os.path.join(PKG, "csrc", "rollout_kernels.cuh"), os.path.join(PKG, "csrc", "policy_kernels.cuh"),
         os.path.join(os.path.dirname(PKG), "include", "swarm_b200.h")]
 LIB_DIR = os.path.join(PKG, "lib")
 LIB = os.path.join(LIB_DIR, "libswarm_b200.so")

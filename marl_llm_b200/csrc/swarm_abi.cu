@@ -4,9 +4,11 @@
 // return SWARM_ERR_NO_DEVICE / SWARM_ERR_CUDA and the legacy (void) calls print the CUDA error and abort.
 #include "swarm_kernels.cuh"
 #include "render_kernels.cuh"
+#include "state_kernels.cuh"
 #include "../../include/swarm_b200.h"
 
 #include <algorithm>
+#include <atomic>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -194,6 +196,7 @@ struct swarm_sim {
     bool all_tables;        // every library shape has a table (a reset cannot leave an env unmatched)
     bool xy_exact;          // every library shape has bit-identical x per lattice column and y per lattice row
     int rec_cap; size_t smem_fast;
+    uint64_t lib_fp;        // fingerprint of the shape library (0: none), see library_fingerprint
 };
 
 // the k_step kernels launch_step runs for one step (dyn) or observe on a scan path (fast: see swarm_fast_path), and their dynamic
@@ -294,6 +297,7 @@ int swarm_create(const swarm_config *cfg, const swarm_buffers *buf, swarm_sim **
     s->d_tabs = nullptr; s->d_pose = nullptr; s->d_shape_id = nullptr;
     s->match.init(cfg->num_envs);
     s->fast_ok = false; s->all_tables = false; s->xy_exact = false; s->rec_cap = 0; s->smem_fast = 0;
+    s->lib_fp = 0;
     {
         cudaError_t e1 = cudaMalloc(&s->d_pose, sizeof(double4) * (size_t)cfg->num_envs);
         cudaError_t e2 = cudaMalloc(&s->d_shape_id, sizeof(int) * (size_t)cfg->num_envs);
@@ -374,7 +378,7 @@ int swarm_set_grid(swarm_sim *s, int32_t env0, int32_t count, const double *grid
     return SWARM_OK;
 }
 
-int swarm_set_shapes(swarm_sim *s, int32_t n_shapes, const double *grids, const int32_t *n_g, const double *l_cell) {
+static int install_shapes(swarm_sim *s, int32_t n_shapes, const double *grids, const int32_t *n_g, const double *l_cell) {
     if (!s || !grids || !n_g || !l_cell || n_shapes <= 0) return fail(SWARM_ERR_INVALID, "bad argument");
     CU_TRY(cudaSetDevice(s->cfg.device));
     const int ngm = s->cfg.n_g_max;
@@ -513,6 +517,36 @@ int swarm_set_shapes(swarm_sim *s, int32_t n_shapes, const double *grids, const 
         if (const int rc = raise_step_smem_limits(s, fast)) return rc;
     s->fast_ok = true;
     return SWARM_OK;
+}
+
+/* What a shape id means on this handle: a hash of the library (shape count, cells, cell sizes) and of which shapes the lookup
+ * scan serves.  A state saved under one fingerprint keeps its match record only when loaded under the same one (DESIGN.md §11). */
+static uint64_t library_fingerprint(const swarm_sim *s, const double *grids, const int32_t *n_g, const double *l_cell) {
+    uint64_t h = 1469598103934665603ull;                                      // FNV-1a
+    auto mix = [&h](const void *p, size_t n) {
+        for (size_t i = 0; i < n; ++i) { h ^= static_cast<const unsigned char *>(p)[i]; h *= 1099511628211ull; }
+    };
+    mix(&s->n_shapes, sizeof(int));
+    for (int k = 0; k < s->n_shapes; ++k) {
+        mix(&n_g[k], sizeof(int32_t)); mix(&l_cell[k], sizeof(double));
+        mix(grids + (size_t)k * 2 * s->cfg.n_g_max, sizeof(double) * 2 * (size_t)n_g[k]);
+        const unsigned char tab = s->h_tabs[k].nb != 0;
+        mix(&tab, 1);
+    }
+    const unsigned char ok = s->fast_ok;
+    mix(&ok, 1);
+    h &= ~(1ull << 63);
+    return h ? h : 1;
+}
+
+int swarm_set_shapes(swarm_sim *s, int32_t n_shapes, const double *grids, const int32_t *n_g, const double *l_cell) {
+    const int rc = install_shapes(s, n_shapes, grids, n_g, l_cell);
+    if (rc == SWARM_OK) s->lib_fp = library_fingerprint(s, grids, n_g, l_cell);
+    else if (rc != SWARM_ERR_INVALID) {        // failed half way: a library no saved state can claim
+        static std::atomic<uint64_t> failed{0};
+        s->lib_fp = (1ull << 63) | ++failed;
+    }
+    return rc;
 }
 
 /* Target shapes for envs [env0, env0 + count) given as (library shape, pose): grid_center = R * origin + off computed on the
@@ -768,6 +802,172 @@ int swarm_restore_observation(swarm_sim *s) {
 }
 
 int swarm_is_observed(const swarm_sim *s) { return (s && s->observed) ? 1 : 0; }
+
+}  // extern "C"
+
+// ---- state store (DESIGN.md §11).  The segments of a slot, in slot order: one env row of each of these arrays.
+enum StateSegId { SEG_P, SEG_DP, SEG_GRID, SEG_WBOX, SEG_FRAME, SEG_NG, SEG_THRESH, SEG_POSE, SEG_SHAPE, SEG_NEAREST, SEG_NBR,
+                  SEG_FLAGS, SEG_OBS, SEG_REWARD, SEG_PRIOR_CUR, SEG_PRIOR_LAST, SEG_SENSED, SEG_OCC, SEG_COUNT };
+static_assert(SEG_COUNT <= STATE_MAX_SEGS, "StateCopyParams::seg too small");
+
+struct swarm_state_store {
+    swarm_config cfg;                         // the configuration it serves (num_envs is not part of it)
+    int64_t capacity;
+    long long row[SEG_COUNT], off[SEG_COUNT]; // bytes per env row (0: not stored) and offset in the slot
+    long long slot_bytes;
+    int n_sm;
+    unsigned char *d_slots;
+    struct Slot {
+        bool filled = false;
+        bool prior_valid = false;             // the source's a_prior[pending] was the prior of its state (!prior_dirty)
+        MatchMirror::State match = MatchMirror::UNMATCHED;   // the source env's mirror entry: never more than the device record
+        uint64_t lib_fp = 0;                  // the source's library_fingerprint
+    };
+    std::vector<Slot> slot;
+};
+
+static bool same_config(const swarm_config &a, const swarm_config &b) {
+    swarm_config x = a, y = b;
+    x.num_envs = y.num_envs = 0;
+    return memcmp(&x, &y, sizeof(swarm_config)) == 0;
+}
+
+// env row e of segment g of the handle starts at state_seg_base(s, g) + e * row[g]
+static unsigned char *state_seg_base(const swarm_sim *s, int g) {
+    const swarm_buffers &b = s->buf;
+    void *const base[SEG_COUNT] = {b.p, b.dp, b.grid, b.word_box, b.frame, b.n_g, b.in_thresh, s->d_pose, s->d_shape_id,
+                                   b.nearest_cell, b.neighbor_index, b.in_flags, b.obs, b.reward, b.a_prior[s->pending],
+                                   b.a_prior[s->last], b.sensed_index, b.occupied_index};
+    return static_cast<unsigned char *>(base[g]);
+}
+
+// checks shared by save and load: handle, store, lists; `distinct` names the list that must not repeat an id
+static int state_check(const swarm_sim *s, const swarm_state_store *st, const int32_t *env_ids, const int32_t *slots, int32_t count,
+                       bool envs_distinct) {
+    if (!s || !st || !env_ids || !slots) return fail(SWARM_ERR_INVALID, "null argument");
+    if (s->cfg.variant != SWARM_VARIANT_ASSEMBLY) return fail(SWARM_ERR_UNSUPPORTED, "the state store serves assembly handles");
+    if (count < 1) return fail(SWARM_ERR_INVALID, "count must be >= 1");
+    if (!same_config(s->cfg, st->cfg)) return fail(SWARM_ERR_INVALID, "the handle's configuration is not the store's");
+    const int E = s->cfg.num_envs;
+    std::vector<char> seen_env(envs_distinct ? E : 0), seen_slot(envs_distinct ? 0 : st->capacity);
+    for (int k = 0; k < count; ++k) {
+        if (env_ids[k] < 0 || env_ids[k] >= E) return fail(SWARM_ERR_INVALID, "env id out of range");
+        if (slots[k] < 0 || slots[k] >= st->capacity) return fail(SWARM_ERR_INVALID, "slot out of range");
+        char &seen = envs_distinct ? seen_env[env_ids[k]] : seen_slot[slots[k]];
+        if (seen) return fail(SWARM_ERR_INVALID, envs_distinct ? "env ids must be distinct" : "slots must be distinct");
+        seen = 1;
+    }
+    return SWARM_OK;
+}
+
+// k_state_copy over the pairs (env_ids[k], slots[k]), STATE_PAIRS_PER_LAUNCH per launch
+static int state_copy(swarm_sim *s, swarm_state_store *st, bool save, const int32_t *env_ids, const int32_t *slots, int32_t count,
+                      cudaStream_t stream) {
+    CU_TRY(cudaSetDevice(s->cfg.device));
+    StateCopyParams P;
+    P.slots = st->d_slots; P.slot_bytes = st->slot_bytes; P.n_segs = 0; P.pad_ = 0;
+    for (int g = 0; g < SEG_COUNT; ++g) {
+        // a handle that has not stepped returns the prior of its current state: a_prior[last] is a_prior[pending]
+        if (!st->row[g] || (!save && g == SEG_PRIOR_LAST && s->last == s->pending)) continue;
+        StateSeg &S = P.seg[P.n_segs++];
+        S.env = state_seg_base(s, g); S.row = st->row[g]; S.off = st->off[g]; S.shape_id = g == SEG_SHAPE; S.pad_ = 0;
+    }
+    for (int k0 = 0; k0 < count; k0 += STATE_PAIRS_PER_LAUNCH) {
+        const int n = std::min(count - k0, STATE_PAIRS_PER_LAUNCH);
+        // at most 32 KB of a slot per CTA, at least 4 KB, and at least two CTAs per SM when the launch carries few pairs
+        const long long sb = st->slot_bytes;
+        long long chunks = std::max((sb + 32767) / 32768, (2LL * st->n_sm + n - 1) / n);
+        chunks = std::min(chunks, (sb + 4095) / 4096);
+        P.chunk = ((sb + chunks - 1) / chunks + 15) & ~15LL;
+        chunks = (sb + P.chunk - 1) / P.chunk;
+        for (int k = 0; k < n; ++k) {
+            const int slot = slots[k0 + k];
+            const bool unmatched = !save && st->slot[slot].lib_fp != s->lib_fp;
+            P.pair[k] = make_int2(env_ids[k0 + k], slot | (unmatched ? STATE_UNMATCHED : 0));
+        }
+        const dim3 grid((unsigned)chunks, (unsigned)n);
+        if (save) k_state_copy<true><<<grid, STATE_THREADS, 0, stream>>>(P);
+        else k_state_copy<false><<<grid, STATE_THREADS, 0, stream>>>(P);
+        CU_TRY(cudaGetLastError());
+        s->launches++;
+    }
+    return SWARM_OK;
+}
+
+extern "C" {
+
+int swarm_state_store_create(const swarm_sim *s, int64_t capacity, swarm_state_store **out) {
+    if (!s || !out) return fail(SWARM_ERR_INVALID, "null argument");
+    if (s->cfg.variant != SWARM_VARIANT_ASSEMBLY) return fail(SWARM_ERR_UNSUPPORTED, "the state store serves assembly handles");
+    if (capacity < 1 || capacity > INT32_MAX) return fail(SWARM_ERR_INVALID, "capacity must be in [1, 2^31)");
+    CU_TRY(cudaSetDevice(s->cfg.device));
+    int n_sm = 0;
+    CU_TRY(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, s->cfg.device));
+    const swarm_config &c = s->cfg;
+    const long long n_a = c.n_a, osz = c.out_dtype == SWARM_F32 ? 4 : 8;
+    long long row[SEG_COUNT] = {};
+    row[SEG_P] = row[SEG_DP] = 2 * n_a * 8;
+    row[SEG_GRID] = (long long)s->K.n_g_pad * 16; row[SEG_WBOX] = (long long)s->K.n_words * 16; row[SEG_FRAME] = 16;
+    row[SEG_NG] = 4; row[SEG_THRESH] = 8; row[SEG_POSE] = sizeof(double4); row[SEG_SHAPE] = 4;
+    row[SEG_NEAREST] = row[SEG_FLAGS] = 4 * n_a; row[SEG_NBR] = 4LL * TOPO * n_a;
+    row[SEG_OBS] = (long long)s->K.obs_dim * n_a * osz; row[SEG_REWARD] = n_a * osz;
+    if (c.want_prior) row[SEG_PRIOR_CUR] = row[SEG_PRIOR_LAST] = 2 * n_a * osz;
+    if (c.emit_indices) { row[SEG_SENSED] = 4LL * c.num_obs_grid_max * n_a; row[SEG_OCC] = 4LL * c.num_occupied_grid_max * n_a; }
+    swarm_state_store *st = new swarm_state_store();
+    st->cfg = c; st->capacity = capacity; st->n_sm = n_sm;
+    long long off = 0;
+    for (int g = 0; g < SEG_COUNT; ++g) { st->row[g] = row[g]; st->off[g] = off; off += (row[g] + 15) & ~15LL; }
+    st->slot_bytes = (off + 127) & ~127LL;
+    st->slot.assign((size_t)capacity, swarm_state_store::Slot{});
+    const cudaError_t e = cudaMalloc(&st->d_slots, (size_t)capacity * st->slot_bytes);
+    if (e != cudaSuccess) {
+        delete st;
+        return fail(SWARM_ERR_CUDA, std::string("cudaMalloc of the state store failed: ") + cudaGetErrorString(e));
+    }
+    *out = st;
+    return SWARM_OK;
+}
+
+int swarm_state_store_destroy(swarm_state_store *st) {
+    if (!st) return SWARM_OK;
+    cudaSetDevice(st->cfg.device);
+    cudaFree(st->d_slots);
+    delete st;
+    return SWARM_OK;
+}
+
+int64_t swarm_state_slot_bytes(const swarm_state_store *st) { return st ? st->slot_bytes : 0; }
+
+int swarm_state_save(swarm_sim *s, swarm_state_store *st, const int32_t *env_ids, const int32_t *slots, int32_t count, void *stream) {
+    if (const int rc = state_check(s, st, env_ids, slots, count, false)) return rc;
+    if (!s->observed) return fail(SWARM_ERR_INVALID, "swarm_state_save needs an observed handle");
+    if (const int rc = state_copy(s, st, true, env_ids, slots, count, (cudaStream_t)stream)) return rc;
+    for (int k = 0; k < count; ++k) {
+        swarm_state_store::Slot &r = st->slot[slots[k]];
+        r.filled = true;
+        r.prior_valid = !s->prior_dirty;
+        r.match = s->match.env[env_ids[k]];
+        r.lib_fp = s->lib_fp;
+    }
+    return SWARM_OK;
+}
+
+int swarm_state_load(swarm_sim *s, swarm_state_store *st, const int32_t *slots, const int32_t *env_ids, int32_t count, void *stream) {
+    if (const int rc = state_check(s, st, env_ids, slots, count, true)) return rc;
+    for (int k = 0; k < count; ++k)
+        if (!st->slot[slots[k]].filled) return fail(SWARM_ERR_INVALID, "slot is empty");
+    if (!s->observed && count != s->cfg.num_envs)
+        return fail(SWARM_ERR_INVALID, "a handle that was never observed can only be loaded as a whole");
+    if (const int rc = state_copy(s, st, false, env_ids, slots, count, (cudaStream_t)stream)) return rc;
+    for (int k = 0; k < count; ++k) {
+        const swarm_state_store::Slot &r = st->slot[slots[k]];
+        // the kernel wrote shape id -1 for a slot of another library: that env is unmatched
+        s->match.set(env_ids[k], r.lib_fp == s->lib_fp ? r.match : MatchMirror::UNMATCHED);
+        if (s->cfg.want_prior && !r.prior_valid) s->prior_dirty = true;     // the next step's k_prior gives the same values
+    }
+    s->observed = true;
+    return SWARM_OK;
+}
 
 static int launch_step(swarm_sim *s, bool dyn, const void *act, int act_dtype, cudaStream_t st, const int32_t *env_list, int32_t count) {
     KParams K = s->K;
