@@ -2,7 +2,7 @@
  * swarm_b200.h — C ABI of the B200-native batched simulator for the MARL-LLM assembly env step path.
  *
  * One shared library (marl_llm_b200/lib/libswarm_b200.so, also reachable as libAssemblyEnv.so)
- * exports these groups of entry points (the first two below; (3)-(5) further down), all `extern "C"`, plain pointers and sizes only:
+ * exports these groups of entry points (the first two below; (3)-(6) further down), all `extern "C"`, plain pointers and sizes only:
  *
  *  (1) LEGACY, stateless, HOST pointers — the five symbols the reference Python env binds with ctypes
  *      (cus_gym/gym/envs/customized_envs/envs_cplus/c_lib.py:11-22 loads build/libAssemblyEnv.so;
@@ -460,6 +460,35 @@ int64_t swarm_state_slot_bytes(const swarm_state_store *st);
  * sim's swarm_launch_count); the caller may free the host arrays when the call returns. */
 int swarm_state_save(swarm_sim *sim, swarm_state_store *st, const int32_t *env_ids, const int32_t *slots, int32_t count, void *stream);
 int swarm_state_load(swarm_sim *sim, swarm_state_store *st, const int32_t *slots, const int32_t *env_ids, int32_t count, void *stream);
+
+/* ============================================================================================
+ * (6) Prior policies as programs (DESIGN.md §12).  A caller's `robot_policy` (include/swarm_prior_api.cuh, which states the
+ *     contract) is compiled at run time into an sm_100a CUBIN and runs as the step's prior (a_prior) or as actions.
+ * ============================================================================================ */
+typedef struct swarm_prior_program swarm_prior_program;   /* opaque: a loaded CUBIN on one device */
+
+/* Host only, no GPU needed: source -> sm_100a CUBIN.  The library appends the entry points of swarm_prior_api.cuh (whose text it
+ * embeds) and compiles with its fixed options --gpu-architecture=sm_100a --fmad=false -default-device (IEEE division and square
+ * root).  NVRTC is opened with dlopen on the first call: nvrtc_path, or libnvrtc.so.12 on the loader path when it is NULL; not
+ * found: SWARM_ERR_UNSUPPORTED, naming the path tried.  Two-call size query: with image = NULL only *image_size is written; then
+ * image_cap >= *image_size bytes at image.  NVRTC's log (errors with their line, warnings) goes to log[log_cap], NUL-terminated
+ * and truncated, when log is non-NULL.  A source that does not compile, or has no robot_policy: SWARM_ERR_INVALID. */
+int swarm_prior_compile(const char *source, const char *nvrtc_path, void *image, int64_t image_cap, int64_t *image_size, char *log,
+                        int64_t log_cap);
+/* Loads a CUBIN of swarm_prior_compile on `device` (cudaLibraryLoadData: no driver JIT).  Destroy a program only after it is
+ * removed from every handle it is installed on. */
+int swarm_prior_program_create(int32_t device, const void *image, int64_t size, swarm_prior_program **out);
+int swarm_prior_program_destroy(swarm_prior_program *prog);
+/* Installs prog as sim's prior: every following swarm_step launches prog's a_prior entry (in the handle's output dtype) on the
+ * pre-step state before the step kernel, which then skips its own prior, and swarm_observe writes no prior.  The nearest cell a
+ * program sees is the one the last observation stored while that observation is of the current state and grid, else it is
+ * scanned.  prog = NULL: the built-in prior again, from the next step on.  Needs want_prior (else SWARM_ERR_INVALID) and an
+ * assembly handle (flocking: SWARM_ERR_UNSUPPORTED); prog on sim's device.  While a program is installed, swarm_state_save records
+ * the slots' prior as stale, so a load into any handle recomputes it. */
+int swarm_set_prior_program(swarm_sim *sim, swarm_prior_program *prog);
+/* prog as the controller (the 'llm' strategy's use of the prior): act_dev [E][2][n_a] f64 (device) from the current state and
+ * the neighbour list of the last observation (sim must be observed).  Legal whether or not sim has want_prior. */
+int swarm_prior_program_actions(swarm_sim *sim, swarm_prior_program *prog, double *act_dev, void *stream);
 
 const char *swarm_last_error(void);
 int swarm_abi_version(void);

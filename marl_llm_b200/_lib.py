@@ -77,7 +77,9 @@ BATCHED_SYMBOLS = ["swarm_grid_pad", "swarm_obs_dim", "swarm_create", "swarm_des
                    "swarm_fill_actions", "swarm_launch_count", "swarm_kernel_geometry", "swarm_last_error",
                    "swarm_abi_version", "swarm_sqrt_threshold", "swarm_debug_rho", "swarm_restore_observation", "swarm_is_observed", "swarm_reset_envs", "swarm_measure_fma_peak", "swarm_fast_path", "swarm_set_grid_pose", "swarm_flock_observe", "swarm_flock_step", "swarm_selftest_division", "swarm_pp_obs_dim", "swarm_pp_observe", "swarm_pp_step",
                    "swarm_render", "swarm_render_palette",
-                   "swarm_state_store_create", "swarm_state_store_destroy", "swarm_state_slot_bytes", "swarm_state_save", "swarm_state_load"]
+                   "swarm_state_store_create", "swarm_state_store_destroy", "swarm_state_slot_bytes", "swarm_state_save", "swarm_state_load",
+                   "swarm_prior_compile", "swarm_prior_program_create", "swarm_prior_program_destroy", "swarm_set_prior_program",
+                   "swarm_prior_program_actions"]
 ROLLOUT_SYMBOLS = ["swarm_rollout_push", "swarm_rollout_gather", "swarm_rollout_push_parts", "swarm_rollout_gather_ring"]
 SWARM_PUSH_OBS, SWARM_PUSH_NEXT_OBS, SWARM_PUSH_SMALL = 1, 2, 4
 POLICY_SYMBOLS = ["swarm_policy_create", "swarm_policy_destroy", "swarm_policy_load", "swarm_policy_step", "swarm_policy_launch_count",
@@ -135,6 +137,11 @@ def load():
     lib.swarm_state_slot_bytes.argtypes = [C.c_void_p]
     lib.swarm_state_save.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]
     lib.swarm_state_load.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]
+    lib.swarm_prior_compile.argtypes = [C.c_char_p, C.c_char_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int64), C.c_char_p, C.c_int64]
+    lib.swarm_prior_program_create.argtypes = [C.c_int32, C.c_void_p, C.c_int64, C.POINTER(C.c_void_p)]
+    lib.swarm_prior_program_destroy.argtypes = [C.c_void_p]
+    lib.swarm_set_prior_program.argtypes = [C.c_void_p, C.c_void_p]
+    lib.swarm_prior_program_actions.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.swarm_set_shapes.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.swarm_reset.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.swarm_reset_envs.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]

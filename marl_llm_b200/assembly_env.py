@@ -56,6 +56,7 @@ class AssemblySwarmEnv:
         self._rend = None
         self.render_traj, self.traj_len = False, 15
         self._grid_dirty = False
+        self._prior_program = None
         self.unwrapped = self
 
     # ---------------------------------------------------------------------------------------- ENV:92-154
@@ -111,11 +112,21 @@ class AssemblySwarmEnv:
             is_periodic=self.is_periodic, d_sen=self.d_sen, size_a=self.size_a, k_ball=float(self.k_ball),
             k_wall=float(self.k_wall), c_wall=float(self.c_wall), dt=self.dt, vel_max=self.Vel_max, mass=float(self.m_a),
             half_width=self.boundary_width_half, half_height=self.boundary_height_half)
+        if self._prior_program is not None:
+            self._sim.set_prior_program(self._prior_program)
         # the shape library (ENV:116-119): grids installed by reset() / by the caller are recognised as rigid transforms of
         # these shapes, which lets the simulator use its lookup-scan kernel (results are identical without it)
         if n_g_cap >= max(self.n_gs):
             self._sim.set_shapes([np.ascontiguousarray(np.asarray(g, dtype=np.float64).T) for g in self.grid_center_origins],
                                  [float(v) for v in self.l_cells])
+
+    def set_prior_program(self, prog):
+        """step()'s fifth output (a_prior, ENV:605-624) from a prior program (marl_llm_b200.prior_program.PriorProgram) instead
+        of the built-in robotPolicy; None restores the built-in one.  Needs training_method 'llm_rl'.  The program stays
+        installed when the env rebuilds its simulator for a larger shape."""
+        if self._sim is not None:
+            self._sim.set_prior_program(prog)
+        self._prior_program = prog
 
     # ---------------------------------------------------------------------------------------- helpers
     def _squeeze(self, a):

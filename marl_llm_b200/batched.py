@@ -126,6 +126,7 @@ class BatchedAssemblySim:
         self.l_cell = np.zeros(E)
         self.n_g = np.zeros(E, dtype=np.int32)
         self.shapes_installed = False
+        self.prior_program = None
 
     # ------------------------------------------------------------------------------------------------
     def close(self):
@@ -254,6 +255,12 @@ class BatchedAssemblySim:
         assert out.is_cuda and out.dtype == torch.float64 and out.is_contiguous() and out.numel() == self.E * 2 * self.n_a
         check(self.lib.swarm_strategy_actions(self._h, k, C.c_void_p(out.data_ptr()), self._stream()), "swarm_strategy_actions")
         return out
+
+    def set_prior_program(self, prog):
+        """Install a prior program (marl_llm_b200.prior_program.PriorProgram): the a_prior of the following steps comes from it.
+        None: the built-in prior again, from the next step on.  The handle keeps a reference to the program."""
+        check(self.lib.swarm_set_prior_program(self._h, prog.handle if prog is not None else None), "swarm_set_prior_program")
+        self.prior_program = prog
 
     def set_obs_buffer(self, obs):
         """Redirect the observation output of the following observe()/step() calls to `obs` (same shape / dtype, CUDA,

@@ -8,12 +8,15 @@ import subprocess
 
 PKG = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(PKG, "csrc", "swarm_abi.cu")
-SRCS = [SRC, os.path.join(PKG, "csrc", "rollout_abi.cu"), os.path.join(PKG, "csrc", "policy_abi.cu")]
+SRCS = [SRC, os.path.join(PKG, "csrc", "rollout_abi.cu"), os.path.join(PKG, "csrc", "policy_abi.cu"), os.path.join(PKG, "csrc", "prior_abi.cu")]
+# the prior-program header is compiled into the library as text (prior_abi.cu hands it to NVRTC): regenerated on every build
+PRIOR_API = os.path.join(os.path.dirname(PKG), "include", "swarm_prior_api.cuh")
 DEPS = SRCS + [os.path.join(PKG, "csrc", "swarm_kernels.cuh"), os.path.join(PKG, "csrc", "render_kernels.cuh"), os.path.join(PKG, "csrc", "state_kernels.cuh"), os.path.join(PKG, "csrc", "rollout_kernels.cuh"), os.path.join(PKG, "csrc", "policy_kernels.cuh"),
-        os.path.join(os.path.dirname(PKG), "include", "swarm_b200.h")]
+        os.path.join(PKG, "csrc", "prior_program.h"), os.path.join(os.path.dirname(PKG), "include", "swarm_b200.h"), PRIOR_API]
 LIB_DIR = os.path.join(PKG, "lib")
 LIB = os.path.join(LIB_DIR, "libswarm_b200.so")
 LEGACY_NAME = os.path.join(LIB_DIR, "libAssemblyEnv.so")
+GEN_DIR = os.path.join(LIB_DIR, "gen")
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",   # B200 only
@@ -37,12 +40,22 @@ def is_stale():
     return any(os.path.getmtime(d) > t for d in DEPS)
 
 
+def write_prior_api_text():
+    """GEN_DIR/swarm_prior_api.inc: the bytes of include/swarm_prior_api.cuh as a C initializer list (prior_abi.cu)."""
+    os.makedirs(GEN_DIR, exist_ok=True)
+    data = open(PRIOR_API, "rb").read()
+    rows = [", ".join(str(b - 256 if b > 127 else b) for b in data[k:k + 32]) for k in range(0, len(data), 32)]   # as signed char
+    with open(os.path.join(GEN_DIR, "swarm_prior_api.inc"), "w") as f:
+        f.write(",\n".join(rows) + "\n")
+
+
 def build_library(force=False, verbose=False):
     if not (force or is_stale()):
         return LIB
     os.makedirs(LIB_DIR, exist_ok=True)
+    write_prior_api_text()
     extra = os.environ.get("SWARM_NVCC_EXTRA", "").split()
-    cmd = [nvcc_path()] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB] + SRCS
+    cmd = [nvcc_path()] + NVCC_FLAGS + ["-I", GEN_DIR] + extra + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB] + SRCS
     env = dict(os.environ)
     env.pop("CC", None); env.pop("CXX", None)        # the image exports a gcc without libgomp specs
     subprocess.check_call(cmd, env=env)

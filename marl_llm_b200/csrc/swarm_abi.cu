@@ -5,6 +5,7 @@
 #include "swarm_kernels.cuh"
 #include "render_kernels.cuh"
 #include "state_kernels.cuh"
+#include "prior_program.h"
 #include "../../include/swarm_b200.h"
 
 #include <algorithm>
@@ -197,6 +198,7 @@ struct swarm_sim {
     bool xy_exact;          // every library shape has bit-identical x per lattice column and y per lattice row
     int rec_cap; size_t smem_fast;
     uint64_t lib_fp;        // fingerprint of the shape library (0: none), see library_fingerprint
+    swarm_prior_program *prior_prog;   // installed prior program (NULL: the built-in prior), DESIGN.md §12
 };
 
 // the k_step kernels launch_step runs for one step (dyn) or observe on a scan path (fast: see swarm_fast_path), and their dynamic
@@ -298,6 +300,7 @@ int swarm_create(const swarm_config *cfg, const swarm_buffers *buf, swarm_sim **
     s->match.init(cfg->num_envs);
     s->fast_ok = false; s->all_tables = false; s->xy_exact = false; s->rec_cap = 0; s->smem_fast = 0;
     s->lib_fp = 0;
+    s->prior_prog = nullptr;
     {
         cudaError_t e1 = cudaMalloc(&s->d_pose, sizeof(double4) * (size_t)cfg->num_envs);
         cudaError_t e2 = cudaMalloc(&s->d_shape_id, sizeof(int) * (size_t)cfg->num_envs);
@@ -945,7 +948,7 @@ int swarm_state_save(swarm_sim *s, swarm_state_store *st, const int32_t *env_ids
     for (int k = 0; k < count; ++k) {
         swarm_state_store::Slot &r = st->slot[slots[k]];
         r.filled = true;
-        r.prior_valid = !s->prior_dirty;
+        r.prior_valid = !s->prior_dirty && !s->prior_prog;     // a program's prior is not the built-in prior of the state
         r.match = s->match.env[env_ids[k]];
         r.lib_fp = s->lib_fp;
     }
@@ -969,9 +972,23 @@ int swarm_state_load(swarm_sim *s, swarm_state_store *st, const int32_t *slots, 
     return SWARM_OK;
 }
 
+// parameters of a prior program's entry points (include/swarm_prior_api.cuh): the nearest cell of the last observation is used
+// while that observation is of the current state and grid, the condition under which the fused prior is used
+static swarm_prior_args prior_args(const swarm_sim *s, void *out) {
+    swarm_prior_args A{};
+    A.n_a = s->cfg.n_a; A.n_g_pad = s->K.n_g_pad; A.stored = !s->prior_dirty;
+    A.p = s->buf.p; A.dp = s->buf.dp; A.grid = s->buf.grid; A.n_g = s->buf.n_g; A.in_thresh = s->buf.in_thresh;
+    A.nbr = s->buf.neighbor_index; A.nearest = s->buf.nearest_cell; A.in_flags = s->buf.in_flags;
+    A.d_sen = s->cfg.d_sen; A.r_avoid = s->cfg.r_avoid; A.size_a = s->cfg.size_a; A.vel_max = s->cfg.vel_max; A.dt = s->cfg.dt;
+    for (int k = 0; k < 4; ++k) A.boundary[k] = s->cfg.boundary_pos[k];
+    A.out = out;
+    return A;
+}
+
 static int launch_step(swarm_sim *s, bool dyn, const void *act, int act_dtype, cudaStream_t st, const int32_t *env_list, int32_t count) {
     KParams K = s->K;
     K.act = act; K.act_f32 = (act_dtype == SWARM_F32);
+    K.want_prior = s->K.want_prior && !s->prior_prog;      // an installed program writes the prior itself (swarm_step)
     K.prior_next = s->buf.a_prior[dyn ? (1 - s->pending) : s->pending];
     K.env_list = env_list;
     const int ctas = env_list ? count : s->cfg.num_envs;
@@ -1071,7 +1088,13 @@ int swarm_step(swarm_sim *s, const void *act, int act_dtype, void *stream) {
     if (!s->observed) return fail(SWARM_ERR_INVALID, "swarm_step before swarm_observe (reset)");
     cudaStream_t st = (cudaStream_t)stream;
     CU_TRY(cudaSetDevice(s->cfg.device));
-    if (s->cfg.want_prior && s->prior_dirty) {
+    if (s->prior_prog) {
+        // the program's prior of the current state (ENV:613-624), in place of the fused prior of the previous step
+        const int entry = s->cfg.out_dtype == SWARM_F32 ? SWARM_PRIOR_F32 : SWARM_PRIOR_F64;
+        if (const int rc = swarm_prior_program_launch_(s->prior_prog, entry, prior_args(s, s->buf.a_prior[s->pending]), s->cfg.num_envs,
+                                                       s->cfg.n_a, st)) return rc;
+        s->launches++;
+    } else if (s->cfg.want_prior && s->prior_dirty) {
         // ENV:613-624 semantics: prior from the current p/dp/grid and the neighbour list of the last observation
         const int n_a = s->cfg.n_a;
         const int th = n_a < 256 ? round32(n_a) : 256;
@@ -1089,6 +1112,29 @@ int swarm_step(swarm_sim *s, const void *act, int act_dtype, void *stream) {
     s->last = s->pending;
     s->pending = 1 - s->pending;
     s->prior_dirty = false;
+    return SWARM_OK;
+}
+
+int swarm_set_prior_program(swarm_sim *s, swarm_prior_program *prog) {
+    if (!s) return fail(SWARM_ERR_INVALID, "null handle");
+    if (s->cfg.variant != SWARM_VARIANT_ASSEMBLY) return fail(SWARM_ERR_UNSUPPORTED, "prior programs serve assembly handles");
+    if (!s->cfg.want_prior) return fail(SWARM_ERR_INVALID, "the handle was created without want_prior: it has no a_prior to write");
+    if (prog && swarm_prior_program_device_(prog) != s->cfg.device) return fail(SWARM_ERR_INVALID, "the program is loaded on another device");
+    // the built-in path again: a_prior[pending] holds no fused prior, so the next step computes it with k_prior
+    if (!prog && s->prior_prog) s->prior_dirty = true;
+    s->prior_prog = prog;
+    return SWARM_OK;
+}
+
+int swarm_prior_program_actions(swarm_sim *s, swarm_prior_program *prog, double *act_dev, void *stream) {
+    if (!s || !prog || !act_dev) return fail(SWARM_ERR_INVALID, "null argument");
+    if (s->cfg.variant != SWARM_VARIANT_ASSEMBLY) return fail(SWARM_ERR_UNSUPPORTED, "prior programs serve assembly handles");
+    if (swarm_prior_program_device_(prog) != s->cfg.device) return fail(SWARM_ERR_INVALID, "the program is loaded on another device");
+    if (!s->observed) return fail(SWARM_ERR_INVALID, "a prior program needs the neighbour list of an observation");
+    CU_TRY(cudaSetDevice(s->cfg.device));
+    if (const int rc = swarm_prior_program_launch_(prog, SWARM_PRIOR_ACTIONS, prior_args(s, act_dev), s->cfg.num_envs, s->cfg.n_a,
+                                                   (cudaStream_t)stream)) return rc;
+    s->launches++;
     return SWARM_OK;
 }
 
