@@ -466,6 +466,7 @@ int swarm_state_load(swarm_sim *sim, swarm_state_store *st, const int32_t *slots
  *     contract) is compiled at run time into an sm_100a CUBIN and runs as the step's prior (a_prior) or as actions.
  * ============================================================================================ */
 typedef struct swarm_prior_program swarm_prior_program;   /* opaque: a loaded CUBIN on one device */
+typedef struct swarm_prior_population swarm_prior_population;   /* opaque: programs and an assignment env -> program */
 
 /* Host only, no GPU needed: source -> sm_100a CUBIN.  The library appends the entry points of swarm_prior_api.cuh (whose text it
  * embeds) and compiles with its fixed options --gpu-architecture=sm_100a --fmad=false -default-device (IEEE division and square
@@ -475,8 +476,9 @@ typedef struct swarm_prior_program swarm_prior_program;   /* opaque: a loaded CU
  * and truncated, when log is non-NULL.  A source that does not compile, or has no robot_policy: SWARM_ERR_INVALID. */
 int swarm_prior_compile(const char *source, const char *nvrtc_path, void *image, int64_t image_cap, int64_t *image_size, char *log,
                         int64_t log_cap);
-/* Loads a CUBIN of swarm_prior_compile on `device` (cudaLibraryLoadData: no driver JIT).  Destroy a program only after it is
- * removed from every handle it is installed on. */
+/* Loads a CUBIN of swarm_prior_compile on `device` (cudaLibraryLoadData: no driver JIT).  Programs and populations are owned by
+ * the caller: destroy a program only after it is removed from every handle it is installed on and every population that lists it
+ * is destroyed, and a population only after it is removed from every handle it is installed on. */
 int swarm_prior_program_create(int32_t device, const void *image, int64_t size, swarm_prior_program **out);
 int swarm_prior_program_destroy(swarm_prior_program *prog);
 /* Installs prog as sim's prior: every following swarm_step launches prog's a_prior entry (in the handle's output dtype) on the
@@ -489,6 +491,26 @@ int swarm_set_prior_program(swarm_sim *sim, swarm_prior_program *prog);
 /* prog as the controller (the 'llm' strategy's use of the prior): act_dev [E][2][n_a] f64 (device) from the current state and
  * the neighbour list of the last observation (sim must be observed).  Legal whether or not sim has want_prior. */
 int swarm_prior_program_actions(swarm_sim *sim, swarm_prior_program *prog, double *act_dev, void *stream);
+/* A population: `count` programs and the program env_program[e] (HOST [num_envs], values in [0, count)) of every env of a handle
+ * with num_envs envs.  Each program runs on its own envs only, so K candidate priors share one batch and one step.  The envs are
+ * grouped by program (ascending env id within a group) and the list is copied once to device memory the population owns (a
+ * synchronous copy).  A program without envs is allowed; it launches nothing.  Checked before anything is allocated
+ * (SWARM_ERR_INVALID, nothing created): count >= 1, num_envs >= 1, no NULL program, every program on `device`, every
+ * env_program[e] in range.  The caller may free both host arrays when the call returns. */
+int swarm_prior_population_create(int32_t device, int32_t num_envs, int32_t count, swarm_prior_program *const *programs,
+                                  const int32_t *env_program, swarm_prior_population **out);
+int swarm_prior_population_destroy(swarm_prior_population *pop);
+/* Installs pop as sim's prior: every following swarm_step launches, in program order, each program's a_prior entry (in the
+ * handle's output dtype) over that program's envs, one launch per program with envs (counted in swarm_launch_count), then the
+ * step kernel without its own prior; otherwise as swarm_set_prior_program.  Installing a population replaces an installed
+ * program, and installing a program replaces a population.  pop = NULL: the built-in prior again, from the next step on.  Needs
+ * want_prior (else SWARM_ERR_INVALID) and an assembly handle (flocking: SWARM_ERR_UNSUPPORTED); pop on sim's device and made for
+ * sim's num_envs (else SWARM_ERR_INVALID).  A rejected call leaves the installed prior in force. */
+int swarm_set_prior_population(swarm_sim *sim, swarm_prior_population *pop);
+/* Every env's program as the controller: act_dev [E][2][n_a] f64 (device), each env's rows written by its program, from the
+ * current state and the neighbour list of the last observation (sim must be observed; pop made for sim's device and num_envs).
+ * Legal whether or not sim has want_prior. */
+int swarm_prior_population_actions(swarm_sim *sim, swarm_prior_population *pop, double *act_dev, void *stream);
 
 const char *swarm_last_error(void);
 int swarm_abi_version(void);

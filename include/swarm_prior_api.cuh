@@ -51,6 +51,7 @@ struct swarm_prior_args {
     double d_sen, r_avoid, size_a, vel_max, dt;
     double boundary[4];
     void *out;                         /* [E][2][n_a] f32 or f64 */
+    const int *env_ids;                /* CTA b serves env env_ids[b] (a population's group); NULL: env b */
 };
 
 #ifdef __CUDACC_RTC__
@@ -101,7 +102,8 @@ struct swarm_agent {
 
 /*
  * Entry points.  swarm_prior_compile appends `#define SWARM_PRIOR_ENTRY` and `#include "swarm_prior_api.cuh"` to the program,
- * so they follow the program's robot_policy.  One CTA per env, threads striding over its agents (the geometry of k_prior):
+ * so they follow the program's robot_policy.  One CTA per env, threads striding over its agents (the geometry of k_prior); with
+ * env_ids, CTA b serves env env_ids[b] and the others are left as they are (a population runs each program on its own envs):
  *   swarm_prior_f32 / swarm_prior_f64   a_prior of the handle, [E][2][n_a] in the output dtype
  *   swarm_prior_actions                  actions [E][2][n_a] f64
  * The nearest cell is the one the last observation stored when that observation is of the current state and grid (stored =
@@ -112,7 +114,7 @@ struct swarm_agent {
 
 template <typename OUT>
 __device__ void swarm_prior_run_(const swarm_prior_args &A) {
-    const int e = blockIdx.x, n_a = A.n_a;
+    const int e = A.env_ids ? A.env_ids[blockIdx.x] : (int)blockIdx.x, n_a = A.n_a;
     const double *pe = A.p + (size_t)e * 2 * n_a, *dpe = A.dp + (size_t)e * 2 * n_a;
     const double *g = A.grid + (size_t)e * A.n_g_pad * 2;
     const int n_g = A.n_g[e];

@@ -79,7 +79,8 @@ BATCHED_SYMBOLS = ["swarm_grid_pad", "swarm_obs_dim", "swarm_create", "swarm_des
                    "swarm_render", "swarm_render_palette",
                    "swarm_state_store_create", "swarm_state_store_destroy", "swarm_state_slot_bytes", "swarm_state_save", "swarm_state_load",
                    "swarm_prior_compile", "swarm_prior_program_create", "swarm_prior_program_destroy", "swarm_set_prior_program",
-                   "swarm_prior_program_actions"]
+                   "swarm_prior_program_actions", "swarm_prior_population_create", "swarm_prior_population_destroy",
+                   "swarm_set_prior_population", "swarm_prior_population_actions"]
 ROLLOUT_SYMBOLS = ["swarm_rollout_push", "swarm_rollout_gather", "swarm_rollout_push_parts", "swarm_rollout_gather_ring"]
 SWARM_PUSH_OBS, SWARM_PUSH_NEXT_OBS, SWARM_PUSH_SMALL = 1, 2, 4
 POLICY_SYMBOLS = ["swarm_policy_create", "swarm_policy_destroy", "swarm_policy_load", "swarm_policy_step", "swarm_policy_launch_count",
@@ -142,6 +143,10 @@ def load():
     lib.swarm_prior_program_destroy.argtypes = [C.c_void_p]
     lib.swarm_set_prior_program.argtypes = [C.c_void_p, C.c_void_p]
     lib.swarm_prior_program_actions.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.swarm_prior_population_create.argtypes = [C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]
+    lib.swarm_prior_population_destroy.argtypes = [C.c_void_p]
+    lib.swarm_set_prior_population.argtypes = [C.c_void_p, C.c_void_p]
+    lib.swarm_prior_population_actions.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.swarm_set_shapes.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.swarm_reset.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.swarm_reset_envs.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]

@@ -127,6 +127,7 @@ class BatchedAssemblySim:
         self.n_g = np.zeros(E, dtype=np.int32)
         self.shapes_installed = False
         self.prior_program = None
+        self.prior_population = None
 
     # ------------------------------------------------------------------------------------------------
     def close(self):
@@ -261,6 +262,15 @@ class BatchedAssemblySim:
         None: the built-in prior again, from the next step on.  The handle keeps a reference to the program."""
         check(self.lib.swarm_set_prior_program(self._h, prog.handle if prog is not None else None), "swarm_set_prior_program")
         self.prior_program = prog
+        self.prior_population = None
+
+    def set_prior_population(self, pop):
+        """Install a prior population (marl_llm_b200.prior_program.PriorPopulation, made for this handle's E): env e's a_prior
+        of the following steps comes from its own program.  Replaces an installed program.  None: the built-in prior again,
+        from the next step on.  The handle keeps a reference to the population."""
+        check(self.lib.swarm_set_prior_population(self._h, pop.handle if pop is not None else None), "swarm_set_prior_population")
+        self.prior_population = pop
+        self.prior_program = None
 
     def set_obs_buffer(self, obs):
         """Redirect the observation output of the following observe()/step() calls to `obs` (same shape / dtype, CUDA,

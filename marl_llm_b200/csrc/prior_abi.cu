@@ -115,13 +115,37 @@ struct swarm_prior_program {
 
 int swarm_prior_program_device_(const swarm_prior_program *prog) { return prog->device; }
 
-int swarm_prior_program_launch_(const swarm_prior_program *prog, int entry, const swarm_prior_args &args, int num_envs, int n_a,
-                                cudaStream_t stream) {
+int swarm_prior_program_launch_(const swarm_prior_program *prog, int entry, const swarm_prior_args &args, const int *env_ids,
+                                int ctas, int n_a, cudaStream_t stream) {
     const int threads = n_a < 256 ? (n_a + 31) & ~31 : 256;          // k_prior's geometry
     swarm_prior_args a = args;
+    a.env_ids = env_ids;
     void *params[] = {&a};
-    const cudaError_t e = cudaLaunchKernel((const void *)prog->entry[entry], dim3(num_envs), dim3(threads), params, 0, stream);
+    const cudaError_t e = cudaLaunchKernel((const void *)prog->entry[entry], dim3(ctas), dim3(threads), params, 0, stream);
     if (e != cudaSuccess) return qfail(SWARM_ERR_CUDA, std::string("prior program launch: ") + cudaGetErrorString(e));
+    return SWARM_OK;
+}
+
+// K programs and an assignment env -> program.  The env ids, grouped by program and ascending within a group, are one device
+// array; program k serves the slice [offset[k], offset[k] + count[k]) of it.
+struct swarm_prior_population {
+    int device, num_envs;
+    std::vector<swarm_prior_program *> prog;
+    std::vector<int> offset, count;
+    int *d_env;
+};
+
+int swarm_prior_population_device_(const swarm_prior_population *pop) { return pop->device; }
+int swarm_prior_population_envs_(const swarm_prior_population *pop) { return pop->num_envs; }
+
+int swarm_prior_population_launch_(const swarm_prior_population *pop, int entry, const swarm_prior_args &args, int n_a,
+                                   cudaStream_t stream, int64_t *launches) {
+    for (size_t k = 0; k < pop->prog.size(); ++k) {
+        if (pop->count[k] == 0) continue;
+        if (const int rc = swarm_prior_program_launch_(pop->prog[k], entry, args, pop->d_env + pop->offset[k], pop->count[k], n_a, stream))
+            return rc;
+        ++*launches;
+    }
     return SWARM_OK;
 }
 
@@ -181,6 +205,51 @@ int swarm_prior_program_destroy(swarm_prior_program *prog) {
     cudaSetDevice(prog->device);
     cudaLibraryUnload(prog->lib);
     delete prog;
+    return SWARM_OK;
+}
+
+int swarm_prior_population_create(int32_t device, int32_t num_envs, int32_t count, swarm_prior_program *const *programs,
+                                  const int32_t *env_program, swarm_prior_population **out) {
+    if (!programs || !env_program || !out) return qfail(SWARM_ERR_INVALID, "null argument");
+    if (count < 1) return qfail(SWARM_ERR_INVALID, "a population needs count >= 1 programs");
+    if (num_envs < 1) return qfail(SWARM_ERR_INVALID, "a population needs num_envs >= 1");
+    for (int k = 0; k < count; ++k) {
+        if (!programs[k]) return qfail(SWARM_ERR_INVALID, "program " + std::to_string(k) + " is NULL");
+        if (programs[k]->device != device) return qfail(SWARM_ERR_INVALID, "program " + std::to_string(k) + " is loaded on another device");
+    }
+    std::vector<int> cnt(count, 0);
+    for (int e = 0; e < num_envs; ++e) {
+        if (env_program[e] < 0 || env_program[e] >= count)
+            return qfail(SWARM_ERR_INVALID, "env_program[" + std::to_string(e) + "] = " + std::to_string(env_program[e]) + " is not in [0, count)");
+        cnt[env_program[e]]++;
+    }
+    std::vector<int> off(count, 0), grouped(num_envs);
+    for (int k = 1; k < count; ++k) off[k] = off[k - 1] + cnt[k - 1];
+    std::vector<int> fill = off;
+    for (int e = 0; e < num_envs; ++e) grouped[fill[env_program[e]]++] = e;
+    cudaError_t err = cudaSetDevice(device);
+    if (err != cudaSuccess) return qfail(SWARM_ERR_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(err));
+    int *d_env = nullptr;
+    err = cudaMalloc(&d_env, sizeof(int) * (size_t)num_envs);
+    if (err == cudaSuccess) err = cudaMemcpy(d_env, grouped.data(), sizeof(int) * (size_t)num_envs, cudaMemcpyHostToDevice);
+    if (err != cudaSuccess) {
+        if (d_env) cudaFree(d_env);
+        return qfail(SWARM_ERR_CUDA, std::string("prior population env list: ") + cudaGetErrorString(err));
+    }
+    swarm_prior_population *pop = new swarm_prior_population();
+    pop->device = device; pop->num_envs = num_envs;
+    pop->prog.assign(programs, programs + count);
+    pop->offset = off; pop->count = cnt;
+    pop->d_env = d_env;
+    *out = pop;
+    return SWARM_OK;
+}
+
+int swarm_prior_population_destroy(swarm_prior_population *pop) {
+    if (!pop) return SWARM_OK;
+    cudaSetDevice(pop->device);
+    cudaFree(pop->d_env);
+    delete pop;
     return SWARM_OK;
 }
 

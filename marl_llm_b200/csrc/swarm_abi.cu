@@ -199,7 +199,11 @@ struct swarm_sim {
     int rec_cap; size_t smem_fast;
     uint64_t lib_fp;        // fingerprint of the shape library (0: none), see library_fingerprint
     swarm_prior_program *prior_prog;   // installed prior program (NULL: the built-in prior), DESIGN.md §12
+    swarm_prior_population *prior_pop; // installed population (NULL: none); at most one of prior_prog and prior_pop is set
 };
+
+// a program or a population writes the prior (swarm_step), not the step kernel or k_prior
+static bool prior_program_installed(const swarm_sim *s) { return s->prior_prog || s->prior_pop; }
 
 // the k_step kernels launch_step runs for one step (dyn) or observe on a scan path (fast: see swarm_fast_path), and their dynamic
 // shared memory; k1 = nullptr when the step is one launch.  The shared-memory limits are raised for exactly these kernels.
@@ -300,7 +304,7 @@ int swarm_create(const swarm_config *cfg, const swarm_buffers *buf, swarm_sim **
     s->match.init(cfg->num_envs);
     s->fast_ok = false; s->all_tables = false; s->xy_exact = false; s->rec_cap = 0; s->smem_fast = 0;
     s->lib_fp = 0;
-    s->prior_prog = nullptr;
+    s->prior_prog = nullptr; s->prior_pop = nullptr;
     {
         cudaError_t e1 = cudaMalloc(&s->d_pose, sizeof(double4) * (size_t)cfg->num_envs);
         cudaError_t e2 = cudaMalloc(&s->d_shape_id, sizeof(int) * (size_t)cfg->num_envs);
@@ -948,7 +952,7 @@ int swarm_state_save(swarm_sim *s, swarm_state_store *st, const int32_t *env_ids
     for (int k = 0; k < count; ++k) {
         swarm_state_store::Slot &r = st->slot[slots[k]];
         r.filled = true;
-        r.prior_valid = !s->prior_dirty && !s->prior_prog;     // a program's prior is not the built-in prior of the state
+        r.prior_valid = !s->prior_dirty && !prior_program_installed(s);   // a program's prior is not the built-in prior of the state
         r.match = s->match.env[env_ids[k]];
         r.lib_fp = s->lib_fp;
     }
@@ -988,7 +992,7 @@ static swarm_prior_args prior_args(const swarm_sim *s, void *out) {
 static int launch_step(swarm_sim *s, bool dyn, const void *act, int act_dtype, cudaStream_t st, const int32_t *env_list, int32_t count) {
     KParams K = s->K;
     K.act = act; K.act_f32 = (act_dtype == SWARM_F32);
-    K.want_prior = s->K.want_prior && !s->prior_prog;      // an installed program writes the prior itself (swarm_step)
+    K.want_prior = s->K.want_prior && !prior_program_installed(s);      // an installed program writes the prior itself (swarm_step)
     K.prior_next = s->buf.a_prior[dyn ? (1 - s->pending) : s->pending];
     K.env_list = env_list;
     const int ctas = env_list ? count : s->cfg.num_envs;
@@ -1088,12 +1092,16 @@ int swarm_step(swarm_sim *s, const void *act, int act_dtype, void *stream) {
     if (!s->observed) return fail(SWARM_ERR_INVALID, "swarm_step before swarm_observe (reset)");
     cudaStream_t st = (cudaStream_t)stream;
     CU_TRY(cudaSetDevice(s->cfg.device));
-    if (s->prior_prog) {
+    if (prior_program_installed(s)) {
         // the program's prior of the current state (ENV:613-624), in place of the fused prior of the previous step
         const int entry = s->cfg.out_dtype == SWARM_F32 ? SWARM_PRIOR_F32 : SWARM_PRIOR_F64;
-        if (const int rc = swarm_prior_program_launch_(s->prior_prog, entry, prior_args(s, s->buf.a_prior[s->pending]), s->cfg.num_envs,
-                                                       s->cfg.n_a, st)) return rc;
-        s->launches++;
+        const swarm_prior_args A = prior_args(s, s->buf.a_prior[s->pending]);
+        if (s->prior_pop) {
+            if (const int rc = swarm_prior_population_launch_(s->prior_pop, entry, A, s->cfg.n_a, st, &s->launches)) return rc;
+        } else {
+            if (const int rc = swarm_prior_program_launch_(s->prior_prog, entry, A, nullptr, s->cfg.num_envs, s->cfg.n_a, st)) return rc;
+            s->launches++;
+        }
     } else if (s->cfg.want_prior && s->prior_dirty) {
         // ENV:613-624 semantics: prior from the current p/dp/grid and the neighbour list of the last observation
         const int n_a = s->cfg.n_a;
@@ -1121,8 +1129,20 @@ int swarm_set_prior_program(swarm_sim *s, swarm_prior_program *prog) {
     if (!s->cfg.want_prior) return fail(SWARM_ERR_INVALID, "the handle was created without want_prior: it has no a_prior to write");
     if (prog && swarm_prior_program_device_(prog) != s->cfg.device) return fail(SWARM_ERR_INVALID, "the program is loaded on another device");
     // the built-in path again: a_prior[pending] holds no fused prior, so the next step computes it with k_prior
-    if (!prog && s->prior_prog) s->prior_dirty = true;
-    s->prior_prog = prog;
+    if (!prog && prior_program_installed(s)) s->prior_dirty = true;
+    s->prior_prog = prog; s->prior_pop = nullptr;
+    return SWARM_OK;
+}
+
+int swarm_set_prior_population(swarm_sim *s, swarm_prior_population *pop) {
+    if (!s) return fail(SWARM_ERR_INVALID, "null handle");
+    if (s->cfg.variant != SWARM_VARIANT_ASSEMBLY) return fail(SWARM_ERR_UNSUPPORTED, "prior programs serve assembly handles");
+    if (!s->cfg.want_prior) return fail(SWARM_ERR_INVALID, "the handle was created without want_prior: it has no a_prior to write");
+    if (pop && swarm_prior_population_device_(pop) != s->cfg.device) return fail(SWARM_ERR_INVALID, "the population is on another device");
+    if (pop && swarm_prior_population_envs_(pop) != s->cfg.num_envs)
+        return fail(SWARM_ERR_INVALID, "the population was made for another number of envs");
+    if (!pop && prior_program_installed(s)) s->prior_dirty = true;
+    s->prior_pop = pop; s->prior_prog = nullptr;
     return SWARM_OK;
 }
 
@@ -1132,10 +1152,20 @@ int swarm_prior_program_actions(swarm_sim *s, swarm_prior_program *prog, double 
     if (swarm_prior_program_device_(prog) != s->cfg.device) return fail(SWARM_ERR_INVALID, "the program is loaded on another device");
     if (!s->observed) return fail(SWARM_ERR_INVALID, "a prior program needs the neighbour list of an observation");
     CU_TRY(cudaSetDevice(s->cfg.device));
-    if (const int rc = swarm_prior_program_launch_(prog, SWARM_PRIOR_ACTIONS, prior_args(s, act_dev), s->cfg.num_envs, s->cfg.n_a,
-                                                   (cudaStream_t)stream)) return rc;
+    if (const int rc = swarm_prior_program_launch_(prog, SWARM_PRIOR_ACTIONS, prior_args(s, act_dev), nullptr, s->cfg.num_envs,
+                                                   s->cfg.n_a, (cudaStream_t)stream)) return rc;
     s->launches++;
     return SWARM_OK;
+}
+
+int swarm_prior_population_actions(swarm_sim *s, swarm_prior_population *pop, double *act_dev, void *stream) {
+    if (!s || !pop || !act_dev) return fail(SWARM_ERR_INVALID, "null argument");
+    if (s->cfg.variant != SWARM_VARIANT_ASSEMBLY) return fail(SWARM_ERR_UNSUPPORTED, "prior programs serve assembly handles");
+    if (swarm_prior_population_device_(pop) != s->cfg.device) return fail(SWARM_ERR_INVALID, "the population is on another device");
+    if (swarm_prior_population_envs_(pop) != s->cfg.num_envs) return fail(SWARM_ERR_INVALID, "the population was made for another number of envs");
+    if (!s->observed) return fail(SWARM_ERR_INVALID, "a prior program needs the neighbour list of an observation");
+    CU_TRY(cudaSetDevice(s->cfg.device));
+    return swarm_prior_population_launch_(pop, SWARM_PRIOR_ACTIONS, prior_args(s, act_dev), s->cfg.n_a, (cudaStream_t)stream, &s->launches);
 }
 
 void *swarm_a_prior_ptr(swarm_sim *s) { return s ? s->buf.a_prior[s->last] : nullptr; }
